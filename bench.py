@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torch.distributed.run)
     python bench.py --impl reference ...                      (the reference's CPU implementation of the path)
+    python bench.py ... --dump-outputs DIR                    (also writes the last timed step's output to DIR/v_out.npy)
 
 metric   : DDIM-50 patch-volumes / s  (one patch-volume = (1,1,8,192,192) thick -> (1,1,48,192,192) thin:
            VAE encode + depth upsample + 51 U-Net evaluations + VAE decode)
@@ -31,6 +32,7 @@ METRIC, UNIT = "ddim50_patch_volumes_per_sec", "patch-volumes/s"
 # algorithmic work per patch-volume (BASELINE.md section 2, measured on the unmodified reference)
 TF_PER_VOLUME = 250.7
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
 
 
 def load_cfg():
@@ -54,6 +56,21 @@ def peaks():
 def synthetic_input(batch, seed=1234):
     g = torch.Generator().manual_seed(seed)
     return torch.rand((batch, 1, T_IN, HW, HW), generator=g) * 2 - 1
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy in float32, so that two builds run with the same arguments can be
+    compared output for output.  An array larger than its share of DUMP_BYTES is written as a fixed sample of its
+    flattened elements: sorted distinct indices drawn with numpy seed 0, which depend on the element count only."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    limit = (DUMP_BYTES // len(arrays) - 4096) // 4  # elements per array; 4096 bytes cover the .npy header
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if a.numel() > limit:
+            idx = torch.unique(torch.from_numpy(np.random.default_rng(0).integers(0, a.numel(), limit)))  # sorted
+            a = a.reshape(-1)[idx.to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 class ClockSampler(threading.Thread):
@@ -330,13 +347,15 @@ def run_gpu(args, rank, world, local_rank):
         host_out.copy_(v, non_blocking=True)  # this rank's slabs; the gathered copy stays on the device for the consumer
 
     def timed(fn, steps):
+        """milliseconds for `steps` calls of fn, and what the last call returned"""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):  # results dropped at once, so only the last one stays allocated
             fn()
+        last = fn()
         gatherer.finish()  # every outstanding gather completes inside the timed region
         e1.record()
         torch.cuda.synchronize()
@@ -345,7 +364,7 @@ def run_gpu(args, rank, world, local_rank):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = t.item()
-        return ms
+        return ms, last
 
     torch.manual_seed(42)
     for _ in range(args.warmup):
@@ -355,17 +374,20 @@ def run_gpu(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     launches0 = _lib.launch_count()
-    ms = timed(step_resident, args.steps)
+    ms, v_out = timed(step_resident, args.steps)
     launches = _lib.launch_count() - launches0
     clocks = sampler.finish() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the e2e steps' gathers reuse v_out's buffer
+        dump_outputs(args.dump_outputs, {"v_out": v_out})
+    del v_out
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     # per-step U-Net time as the sampler runs it: the DDIM loop alone (51 graph replays incl. the scheduler update)
     from v2v_b200.inference import DDIMSampler
     lat = (BATCH, 8, T_OUT, HW // 4, HW // 4)
     cond = torch.randn(lat, device=dev)
     ddim = DDIMSampler(model.diffusion, model.unet)
-    ms_loop = timed(lambda: ddim.sample(lat, cond, DDIM_STEPS, dev, progress=False), 2) / 2
+    ms_loop = timed(lambda: ddim.sample(lat, cond, DDIM_STEPS, dev, progress=False), 2)[0] / 2
     if rank != 0:
         return
     pk = peaks()
@@ -466,8 +488,9 @@ def run_workload(args, rank, world, local_rank):
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
@@ -475,7 +498,7 @@ def run_workload(args, rank, world, local_rank):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = t.item()
-        return ms
+        return ms, last
 
     if w in ("config1", "config3"):
         for _ in range(args.warmup):
@@ -487,11 +510,13 @@ def run_workload(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     n0 = _lib.launch_count()
-    ms = timed(args.steps)
+    ms, v_out = timed(args.steps)
     launches = _lib.launch_count() - n0
     clocks = sampler.finish() if rank == 0 else None
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"v_out": v_out})
     pk = peaks()
     value = units * args.steps / (ms / 1e3)
     tf = {"config4": 4443.6}.get(w, TF_PER_VOLUME)
@@ -518,7 +543,14 @@ def main():
                     help="--impl reference: run only steps + warmup DDIM iterations and extrapolate the loop")
     ap.add_argument("--workload", default="config2", choices=["config1", "config2", "config3", "config4", "config5"],
                     help="BASELINE.json configuration; the default (configs[1]) is the headline line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/v_out.npy (float32; an output over 64 MB is "
+                         "written as a fixed seeded sample of its flattened elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -23,7 +23,15 @@ def test_c_abi_exports_every_declared_symbol():
     assert not missing, missing
     assert set(_lib.SIGNATURES) == declared  # the ctypes binding covers the whole header, and nothing else
     L = _lib.lib()
-    assert L.b2v_abi_version() == 2 and L.b2v_launch_count() == 0
+    assert L.b2v_abi_version() == 2
+    # a freshly loaded library has launched nothing; checked in a new process, since GPU tests run earlier in this one
+    # launch kernels through the same handle
+    import subprocess
+    import sys
+    probe = (f"import sys; sys.path.insert(0, {ROOT!r}); from v2v_b200 import _lib; L = _lib.lib(); "
+             "print(L.b2v_abi_version(), L.b2v_launch_count())")
+    r = subprocess.run([sys.executable, "-c", probe], capture_output=True, text=True)
+    assert r.stdout.split() == ["2", "0"], (r.stdout, r.stderr)
 
 
 def test_c_abi_has_no_torch_or_cpu_fallback_dependency():
