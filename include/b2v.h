@@ -42,7 +42,8 @@ typedef struct {
   int num_levels;
   int channel_mult[8];
   int attention_mask; /* bit l set <=> level l has TemporalAttention (attention_levels) */
-  int num_heads;      /* accepted for parity; the reference's attention output does not depend on it (see DESIGN.md) */
+  int num_heads;      /* reference attention mode: accepted for parity, the output does not depend on it (see DESIGN.md);
+                         softmax mode: the number of heads, head_dim = channels / num_heads                          */
   int time_embed_dim;
 } b2v_unet_desc;
 
@@ -50,6 +51,14 @@ int b2v_unet_create(b2v_unet** out, const b2v_unet_desc* desc);
 void b2v_unet_destroy(b2v_unet* u);
 /* state_dict entry by its reference key (e.g. "down_blocks.0.0.0.conv1.conv.weight"); data = HOST fp32, copied */
 int b2v_unet_load_weight(b2v_unet* u, const char* key, const float* data, const int64_t* shape, int ndim);
+/* TemporalAttention semantics, between create and finalize:
+ *   0 = reference (default): the reference's 'bhqk,bhvc->bhqc' contraction (models/unet3d.py:185), whose output does not
+ *       depend on q, k or the softmax; executed as the folded x + Wp*(Wv*sum_t GN(x) + T*bv) + bp
+ *   1 = softmax: ordinary attention over the T depth tokens of each spatial position and head,
+ *       x + proj_out(softmax(q k^T / sqrt(head_dim)) v), for checkpoints trained with 'bhqk,bhkc->bhqc';
+ *       head_dim = channels / num_heads of every attention level must be a multiple of 16 in [16, 128]
+ * fails after finalize, for an unknown mode or an unsupported head_dim.  The state_dict keys are the same in both. */
+int b2v_unet_set_attention(b2v_unet* u, int mode);
 /* repack all weights (fp16 K-major tiles, folded attention); fails listing the first missing key */
 int b2v_unet_finalize(b2v_unet* u);
 /* UNet3D.forward (models/unet3d.py:357): x, c: (B,L,T,h,w); t: (B,) int64 device; eps_out: (B,L,T,h,w) */
@@ -197,7 +206,8 @@ int b2v_conv_forward(b2v_conv* c, const void* in0, const void* in1, void* out, i
                      int groups, int act_tanh, int N, int D, int H, int W, void* stream);
 int b2v_nc32_to_cl16(const float* in, void* out, int B, int C, int Cpad, long long S, void* stream);
 int b2v_cl16_to_nc32(const void* in, float* out, int B, int C, int Cpad, long long S, void* stream);
-/* out = silu(gn(y)) + temb (mode 0) or silu(gn(y) + res) (mode 1); stats_in as produced by b2v_conv_forward */
+/* out = silu(gn(y)) + temb (mode 0), silu(gn(y) + res) (mode 1) or gn(y) (mode 2); stats_in as produced by
+ * b2v_conv_forward */
 int b2v_gn_apply(const void* y, void* out, const int64_t* stats_in, const float* gamma, const float* beta,
                  const float* temb, const void* res, int B, long long S, int C, int G, int mode, int64_t* stats_out,
                  int G_out, void* stream);
@@ -210,6 +220,10 @@ int b2v_gn_stats(const void* x, int B, long long S, int C, int G, int64_t* stats
 int b2v_res_attn_tail(void* y, const void* res, const int64_t* stats_in, const float* gamma2, const float* beta2, int G2,
                       const float* gamma_a, const float* beta_a, int Ga, const void* wt, const float* bias,
                       int64_t* stats_mid, float* tsum_ws, long long tsum_cap, int B, int T, int P, int C, void* stream);
+/* softmax temporal attention (the U-Net's softmax mode): qkv = cl16 [B][T][P][3C] (the qkv 1x1 conv output; q, k, v
+ * of head h are channels h*hd, C + h*hd, 2C + h*hd, hd = C / heads), out = cl16 [B][T][P][C] with
+ * out[b, :, p, h*hd:(h+1)*hd] = softmax(q k^T / sqrt(hd)) v over the T tokens; hd a multiple of 16 in [16, 128]      */
+int b2v_temporal_attention(const void* qkv, void* out, int B, int T, int P, int C, int heads, void* stream);
 /* DDIM update of one step, coef = device fp32[8] {c1,c2,c3,c4,sigma,..} (inference/sampler.py:299-329) */
 int b2v_ddim_update(float* z, const float* eps, const float* noise, const float* coef, long long n, int* nan_flag,
                     void* stream);

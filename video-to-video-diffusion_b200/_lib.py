@@ -47,6 +47,7 @@ SIGNATURES = {
     "b2v_unet_create": (c_int, [POINTER(_P), POINTER(UNetDesc)]),
     "b2v_unet_destroy": (None, [_P]),
     "b2v_unet_load_weight": (c_int, [_P, c_char_p, _P, POINTER(c_int64), c_int]),
+    "b2v_unet_set_attention": (c_int, [_P, c_int]),
     "b2v_unet_finalize": (c_int, [_P]),
     "b2v_unet_forward": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P]),
     "b2v_ddim_sample": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, POINTER(c_int64), c_int, POINTER(c_float),
@@ -87,6 +88,7 @@ SIGNATURES = {
     "b2v_gn_apply": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_longlong, c_int, c_int, c_int, _P, c_int, _P]),
     "b2v_res_attn_tail": (c_int, [_P, _P, _P, _P, _P, c_int, _P, _P, c_int, _P, _P, _P, _P, c_longlong, c_int, c_int,
                                   c_int, c_int, _P]),
+    "b2v_temporal_attention": (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P]),
     "b2v_gn_stats": (c_int, [_P, c_int, c_longlong, c_int, c_int, _P, _P]),
     "b2v_ddim_update": (c_int, [_P, _P, _P, _P, c_longlong, _P, _P]),
     "b2v_ddpm_update": (c_int, [_P, _P, _P, POINTER(c_float), c_longlong, _P]),

@@ -77,6 +77,10 @@ int b2v_unet_load_weight(b2v_unet* u, const char* key, const float* data, const 
   if (!u) return fail("unet_load_weight: null handle");
   return store_weight(u->u.wm, u->u.finalized, key, data, shape, ndim);
 }
+int b2v_unet_set_attention(b2v_unet* u, int mode) {
+  if (!u) return fail("unet_set_attention: null handle");
+  return u->u.set_attention(mode);
+}
 int b2v_unet_finalize(b2v_unet* u) {
   if (!u) return fail("unet_finalize: null handle");
   return u->u.finalize();
@@ -403,6 +407,7 @@ int b2v_gn_apply(const void* y, void* out, const int64_t* stats_in, const float*
                  const float* temb, const void* res, int B, long long S, int C, int G, int mode, int64_t* stats_out,
                  int G_out, void* stream) {
   if (C % 8 || C / 8 > 256) return fail("gn_apply: C must be a multiple of 8 and <= 2048");
+  if (mode < 0 || mode > 2) return fail("gn_apply: mode must be 0, 1 or 2");
   launch_gn_apply((const __half*)y, (__half*)out, (const stat_t*)stats_in, gamma, beta, temb, C, (const __half*)res, B, S,
                   C, G, 1e-5f, mode, (stat_t*)stats_out, G_out, (cudaStream_t)stream, nullptr, 0);
   g_launches += 1;
@@ -427,6 +432,16 @@ int b2v_res_attn_tail(void* y, const void* res, const int64_t* stats_in, const f
   g_launches += 3;
   B2V_CUDA(cudaGetLastError());
   return 0;
+}
+int b2v_temporal_attention(const void* qkv, void* out, int B, int T, int P, int C, int heads, void* stream) {
+  if (check_device()) return -1;
+  if (!qkv || !out) return fail("temporal_attention: null argument");
+  TAttnPlan plan;
+  std::string err;
+  if (tattn_plan(plan, (const __half*)qkv, (__half*)out, B, T, P, C, heads, err)) return fail(err);
+  tattn_launch(plan, (cudaStream_t)stream);
+  g_launches += 1;
+  return check_launches("temporal_attention");
 }
 int b2v_gn_stats(const void* x, int B, long long S, int C, int G, int64_t* stats, void* stream) {
   launch_gn_stats((const __half*)x, B, S, C, G, (stat_t*)stats, (cudaStream_t)stream);

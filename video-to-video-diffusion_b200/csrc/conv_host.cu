@@ -2,6 +2,7 @@
 
 #include "conv_igemm_t.cuh"
 #include "ew_kernels.h"
+#include "temporal_attention.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -564,6 +565,83 @@ void conv_launch(const ConvPlan& P, cudaStream_t st) {
     case 128: launch_k(conv_igemm_kernel<128>, dim3(P.grid), dim3(ConvCfg<128>::THREADS), ConvCfg<128>::SMEM, st, P.p); break;
     default: launch_k(conv_igemm_kernel<256>, dim3(P.grid), dim3(ConvCfg<256>::THREADS), ConvCfg<256>::SMEM, st, P.p); break;
   }
+}
+
+// ------------------------------------------------------------------ softmax temporal attention (temporal_attention.cuh)
+bool tattn_head_dim_ok(int hd) { return hd >= 16 && hd <= 128 && hd % 16 == 0; }
+
+int tattn_plan(TAttnPlan& P, const __half* qkv, __half* out, int B, int T, int Pn, int C, int heads, std::string& err) {
+  P = TAttnPlan();
+  if (B < 1 || T < 1 || Pn < 1 || heads < 1 || C % heads) {
+    err = "temporal_attention: bad shape (B, T, P >= 1 and C divisible by heads)";
+    return -1;
+  }
+  const int hd = C / heads;
+  if (!tattn_head_dim_ok(hd)) {
+    err = "temporal_attention: head_dim = C / heads = " + std::to_string(hd) +
+          " is not supported (a multiple of 16 in [16, 128])";
+    return -1;
+  }
+  TAttnParams& p = P.p;
+  p.out = out;
+  p.T = T;
+  p.P = Pn;
+  p.C = C;
+  p.heads = heads;
+  p.hd = hd;
+  p.TT = T >= 128 ? 128 : (T + 15) / 16 * 16;
+  p.nkt = (T + p.TT - 1) / p.TT;
+  p.chunks = (hd + 63) / 64;
+  p.pch = (p.TT + 63) / 64;
+  p.units = (long long)B * Pn * heads * p.nkt;
+  p.o_col = (p.TT + 31) / 32 * 32;
+  p.tm_cols = 32;
+  while (p.tm_cols < p.o_col + hd) p.tm_cols *= 2;
+  p.scale_log2 = (float)(1.4426950408889634 / sqrt((double)hd));
+  // shared memory: Q ring, K ring, V ring, P, the overread slack of the M = 128 operand reads, barriers, alignment
+  const size_t CB = (size_t)p.TT * 128, tile = CB * p.chunks;
+  const size_t kMaxSmem = 232448;  // 227 KB per block
+  auto need = [&](int nq, int nkv) {
+    return (nq + 2 * nkv) * tile + p.pch * CB + (size_t)(128 - p.TT) * 128 + 128 + 1024;
+  };
+  const int rings[4][2] = {{2, 2}, {1, 2}, {2, 1}, {1, 1}};
+  int pick = -1;
+  for (int i = 0; i < 4 && pick < 0; ++i)
+    if (need(rings[i][0], rings[i][1]) <= kMaxSmem) pick = i;
+  if (pick < 0) {
+    err = "temporal_attention: tile does not fit in shared memory";
+    return -1;
+  }
+  p.nq = rings[pick][0];
+  p.nkv = rings[pick][1];
+  const size_t smem = need(p.nq, p.nkv);
+  cudaError_t e = cudaFuncSetAttribute(temporal_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
+  int occ = 0;
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, temporal_attention_kernel, TATTN_THREADS, smem);
+  if (e != cudaSuccess) {
+    err = std::string("temporal_attention: ") + cudaGetErrorString(e);
+    return -1;
+  }
+  // co-resident CTAs share the SM's 512 TMEM columns: request enough shared memory that no more than that fit
+  int cps = occ < 512 / p.tm_cols ? occ : 512 / p.tm_cols;
+  if (cps < 1) cps = 1;
+  const size_t fence = 233472 / (size_t)(cps + 1) - 1024 + 128;  // (cps + 1) blocks of this size exceed the SM
+  P.smem = smem > fence ? smem : (fence > kMaxSmem ? kMaxSmem : fence);
+  const long long slots = (long long)device_sm_count() * cps;
+  P.grid = (int)(p.units < slots ? p.units : slots);
+  // (3C, P, T, B) view of the qkv tensor; a box is 64 channels of TT consecutive depths at one position
+  const cuuint64_t C3 = 3 * (cuuint64_t)C;
+  cuuint64_t dims[4] = {C3, (cuuint64_t)Pn, (cuuint64_t)T, (cuuint64_t)B};
+  cuuint64_t strides[3] = {C3 * 2, C3 * Pn * 2, C3 * Pn * T * 2};
+  cuuint32_t box[4] = {64, 1, (cuuint32_t)p.TT, 1};
+  if (encode_map(&p.tm, qkv, 4, dims, strides, box, err)) return -1;
+  P.flops = 4.0 * B * Pn * (double)T * T * C;  // Q K^T and P V
+  P.bytes = (double)B * T * Pn * (3.0 * C + C) * 2.0;
+  return 0;
+}
+
+void tattn_launch(const TAttnPlan& P, cudaStream_t st) {
+  launch_k(temporal_attention_kernel, dim3(P.grid), dim3(TATTN_THREADS), P.smem, st, P.p);
 }
 
 }  // namespace b2v

@@ -85,4 +85,15 @@ int conv_setup_kernels(std::string& err);  // opt-in to large dynamic shared mem
 int device_sm_count();
 __half conv_operand(float x);  // fp32 -> MMA operand (fp16; BF16-rounded first under B2V_OPERANDS=bf16)
 
+// softmax temporal attention (temporal_attention.cuh): qkv NDHWC fp16 [B][T][P][3C] -> out [B][T][P][C]
+struct TAttnPlan {
+  TAttnParams p;
+  int grid = 0;
+  size_t smem = 0;
+  double flops = 0, bytes = 0;  // algorithmic: Q K^T + P V; qkv read once, o written once
+};
+bool tattn_head_dim_ok(int hd);  // a multiple of 16 in [16, 128]
+int tattn_plan(TAttnPlan& P, const __half* qkv, __half* out, int B, int T, int Pn, int C, int heads, std::string& err);
+void tattn_launch(const TAttnPlan& P, cudaStream_t st);
+
 }  // namespace b2v

@@ -29,4 +29,20 @@ struct ConvParams {
   long long ws_slab;      // elements per slab
 };
 
+// softmax temporal attention (temporal_attention.cuh)
+struct TAttnParams {
+  CUtensorMap tm;  // (3C, P, T, B) view of qkv, box (64, 1, TT, 1), 128-byte swizzle
+  void* out;             // __half [B][T][P][C]
+  long long units;
+  int T, P, C, heads, hd;
+  int TT;            // query / key tile rows
+  int nkt;           // key tiles (= query tiles) per (b, position, head)
+  int chunks;        // 64-channel chunks of one head (ceil(hd / 64))
+  int pch;           // 64-key chunks of the P tile (ceil(TT / 64))
+  int nq, nkv;       // depths of the Q and K/V rings (1 or 2)
+  int o_col;         // first TMEM column of O (S occupies columns [0, TT))
+  int tm_cols;       // TMEM columns allocated
+  float scale_log2;  // log2(e) / sqrt(hd)
+};
+
 }  // namespace b2v

@@ -105,6 +105,7 @@ __device__ __forceinline__ void block_stats_out(const float (&as)[8], const floa
 // (models/unet3d.py:70-74,116-133; models/vae.py:31-35,50-56,72-76,93-97), conv_out[0:2] (unet3d.py:328-330).
 //   mode 0: out = silu(gn(y)) + temb[b][c]           (temb may be null)
 //   mode 1: out = silu(gn(y) + res)                  (res may be null)
+//   mode 2: out = gn(y)                              (out of place: the softmax attention block keeps y for its residual)
 // stats_in : [B][G][2] raw (sum, sumsq) over S*cpg elements, produced by the conv epilogue.
 // Grid: (blocks, B); block = C8*R threads, each thread owns 8 fixed channels and strides over rows.
 // ------------------------------------------------------------------------------------------------
@@ -166,6 +167,9 @@ __global__ void __launch_bounds__(256, (!STATS && U <= 4) ? 3 : 2) gn_apply_kern
       if (MODE == 0) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) f[j] = silu_f(f[j] * sc[j] + sh[j]) + ta[j];
+      } else if (MODE == 2) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) f[j] = f[j] * sc[j] + sh[j];
       } else {
         float rf[8];
         if (res) {
@@ -220,6 +224,9 @@ void launch_gn_apply(const __half* y, __half* out, const stat_t* stats_in, const
     if (mode == 0) {                          \
       if (stats_out) GN_LAUNCH(UU, 0, true);  \
       else GN_LAUNCH(UU, 0, false);           \
+    } else if (mode == 2) {                   \
+      if (stats_out) GN_LAUNCH(UU, 2, true);  \
+      else GN_LAUNCH(UU, 2, false);           \
     } else {                                  \
       if (stats_out) GN_LAUNCH(UU, 1, true);  \
       else GN_LAUNCH(UU, 1, false);           \

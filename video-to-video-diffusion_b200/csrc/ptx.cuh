@@ -80,6 +80,19 @@ __device__ __forceinline__ void tma_load_3d(void* smem, const CUtensorMap* m, ui
       : "r"(smem_u32(smem)), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
+__device__ __forceinline__ void tma_load_4d(void* smem, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2,
+                                            int c3) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes"
+      " [%0], [%1, {%3, %4, %5, %6}], [%2];"
+      :
+      : "r"(smem_u32(smem)), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
+// generic-proxy shared-memory writes of this thread become visible to the async proxy (tensor core operand reads)
+__device__ __forceinline__ void fence_proxy_async_smem() {
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
 
 // ---------------------------------------------------------------- tcgen05
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -102,6 +115,17 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) {
   uint64_t d = 0;
   d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
   d |= (uint64_t)1 << 16;
+  d |= (uint64_t)(1024 >> 4) << 32;
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)2 << 61;
+  return d;
+}
+// MN-major, 128-byte-swizzled operand tile: each 128 B row holds 64 consecutive MN elements of one K index, 8-row
+// (8 K) atoms 1024 B apart (SBO); the next 64 MN elements start lbo_bytes further (LBO).
+__device__ __forceinline__ uint64_t umma_desc_sw128_mn(uint32_t saddr, uint32_t lbo_bytes) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
+  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
   d |= (uint64_t)(1024 >> 4) << 32;
   d |= (uint64_t)1 << 46;
   d |= (uint64_t)2 << 61;
@@ -230,6 +254,17 @@ __device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, float* v) {
       : "r"(taddr)
       : "memory");
 }
+// 32 lanes x 16 consecutive fp32 columns, the store counterpart of tmem_ld_32x16
+__device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const float* v) {
+  const uint32_t* r = reinterpret_cast<const uint32_t*>(v);
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
+      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
+      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ---------------------------------------------------------------- programmatic dependent launch
 // Every kernel of the library calls pdl_trigger() (lets the NEXT kernel in the stream start its prologue on SMs

@@ -30,8 +30,10 @@ static int load_res(ResW& r, const WeightMap& wm, const std::string& pre, int ci
   return 0;
 }
 
-// TemporalAttention fold (see ew_kernels.cu: attn_tsum): Wpv = Wp*Wv, u = Wp*bv (bias = T*u + bp at plan time)
-static int load_attn(AttnW& a, const WeightMap& wm, const std::string& pre, int C, DeviceStore& ds) {
+// reference mode: the TemporalAttention fold (see ew_kernels.cu: attn_tsum): Wpv = Wp*Wv, u = Wp*bv (bias = T*u + bp
+// at plan time).  softmax mode: the qkv conv as it is and the output projection as a dual-source conv over (o, x)
+// with weight [Wp | I_C], whose identity half adds the block input into the fp32 accumulator (the residual).
+static int load_attn(AttnW& a, const WeightMap& wm, const std::string& pre, int C, DeviceStore& ds, int mode) {
   a.C = C;
   if (load_gn(a.norm, wm, pre + ".norm", C, groups32(C), ds)) return -1;
   const HostTensor* qkv = need(wm, pre + ".qkv.weight", 3LL * C * C);
@@ -39,6 +41,19 @@ static int load_attn(AttnW& a, const WeightMap& wm, const std::string& pre, int 
   const HostTensor* pw = need(wm, pre + ".proj_out.weight", (long long)C * C);
   const HostTensor* pb = need(wm, pre + ".proj_out.bias", C);
   if (!qkv || !qb || !pw || !pb) return -1;
+  if (mode == ATTN_SOFTMAX) {
+    std::string err;
+    if (conv_layer_init(a.qkv, CONV_K1, qkv->data.data(), qb->data.data(), C, 0, 3 * C, err))
+      return fail(pre + ".qkv: " + err);
+    std::vector<float> wcat((size_t)C * 2 * C, 0.f);  // torch layout [co][ci], ci over cat(o, x)
+    for (int o = 0; o < C; ++o) {
+      for (int i = 0; i < C; ++i) wcat[(size_t)o * 2 * C + i] = pw->data[(size_t)o * C + i];
+      wcat[(size_t)o * 2 * C + C + o] = 1.f;
+    }
+    if (conv_layer_init(a.proj, CONV_K1, wcat.data(), pb->data.data(), C, C, C, err))
+      return fail(pre + ".proj_out: " + err);
+    return 0;
+  }
   const float* Wv = qkv->data.data() + 2LL * C * C;
   const float* bv = qb->data.data() + 2LL * C;
   const float* Wp = pw->data.data();
@@ -69,6 +84,28 @@ static int load_attn(AttnW& a, const WeightMap& wm, const std::string& pre, int 
   a.Wt = (__half*)ds.alloc(wt.size() * sizeof(__half));
   if (!a.Wt || cudaMemcpy(a.Wt, wt.data(), wt.size() * sizeof(__half), cudaMemcpyHostToDevice) != cudaSuccess)
     return fail(pre + ": device alloc failed for the folded attention weights");
+  return 0;
+}
+
+static bool has_attention(const b2v_unet_desc& d, int l) { return (d.attention_mask >> l) & 1; }
+
+int UNet::set_attention(int mode) {
+  if (finalized) return fail("unet_set_attention: the U-Net is already finalized (set the mode before finalize)");
+  if (mode != ATTN_REFERENCE && mode != ATTN_SOFTMAX)
+    return fail("unet_set_attention: unknown mode " + std::to_string(mode) + " (0 = reference, 1 = softmax)");
+  if (mode == ATTN_SOFTMAX) {
+    const b2v_unet_desc& d = desc;
+    if (d.num_heads < 1) return fail("unet_set_attention: softmax attention needs num_heads >= 1");
+    for (int l = 0; l < d.num_levels; ++l) {
+      const int C = d.model_channels * d.channel_mult[l];
+      // every level with attention, and the mid block (at the channel count of the last level)
+      if (!has_attention(d, l) && l != d.num_levels - 1) continue;
+      if (C % d.num_heads || !tattn_head_dim_ok(C / d.num_heads))
+        return fail("unet_set_attention: softmax attention at " + std::to_string(C) + " channels with " +
+                    std::to_string(d.num_heads) + " heads: head_dim must be a multiple of 16 in [16, 128]");
+    }
+  }
+  attention = mode;
   return 0;
 }
 
@@ -113,7 +150,7 @@ int UNet::finalize() {
     for (int i = 0; i < d.num_res_blocks; ++i) {
       const std::string pre = "down_blocks." + std::to_string(l) + "." + std::to_string(i);
       if (load_res(enc[l].res[i], wm, pre + ".0", ch, 0, out_ch, td, ds, pw, pb)) return -1;
-      if (at && load_attn(enc[l].attn[i], wm, pre + ".1", out_ch, ds)) return -1;
+      if (at && load_attn(enc[l].attn[i], wm, pre + ".1", out_ch, ds, attention)) return -1;
       ch = out_ch;
     }
     level_ch[l] = ch;
@@ -123,7 +160,7 @@ int UNet::finalize() {
       return -1;
   }
   if (load_res(mid1, wm, "mid_block1", ch, 0, ch, td, ds, pw, pb)) return -1;
-  if (load_attn(mid_attn, wm, "mid_attn", ch, ds)) return -1;
+  if (load_attn(mid_attn, wm, "mid_attn", ch, ds, attention)) return -1;
   if (load_res(mid2, wm, "mid_block2", ch, 0, ch, td, ds, pw, pb)) return -1;
   dec.resize(NL);
   for (int j = 0; j < NL; ++j) {
@@ -136,7 +173,7 @@ int UNet::finalize() {
       const std::string pre = "up_blocks." + std::to_string(j) + "." + std::to_string(i);
       const int skip_ch = (i == 0) ? mc * d.channel_mult[lvl] : 0;  // models/unet3d.py:303-306
       if (load_res(dec[j].res[i], wm, pre + ".0", ch, skip_ch, out_ch, td, ds, pw, pb)) return -1;
-      if (at && load_attn(dec[j].attn[i], wm, pre + ".1", out_ch, ds)) return -1;
+      if (at && load_attn(dec[j].attn[i], wm, pre + ".1", out_ch, ds, attention)) return -1;
       ch = out_ch;
     }
     dec[j].has_resample = (j < NL - 1);
@@ -157,6 +194,11 @@ int UNet::finalize() {
 
 UNet::~UNet() {
   progs.clear();
+  auto fa = [](AttnW& a) {
+    conv_layer_free(a.pv);
+    conv_layer_free(a.qkv);
+    conv_layer_free(a.proj);
+  };
   auto fr = [](ResW& r) {
     conv_layer_free(r.conv1);
     conv_layer_free(r.conv2);
@@ -164,17 +206,17 @@ UNet::~UNet() {
   };
   for (auto& lv : enc) {
     for (auto& r : lv.res) fr(r);
-    for (auto& a : lv.attn) conv_layer_free(a.pv);
+    for (auto& a : lv.attn) fa(a);
     conv_layer_free(lv.resample);
   }
   for (auto& lv : dec) {
     for (auto& r : lv.res) fr(r);
-    for (auto& a : lv.attn) conv_layer_free(a.pv);
+    for (auto& a : lv.attn) fa(a);
     conv_layer_free(lv.resample);
   }
   fr(mid1);
   fr(mid2);
-  conv_layer_free(mid_attn.pv);
+  fa(mid_attn);
   conv_layer_free(conv_in);
   conv_layer_free(conv_out);
 }
@@ -241,6 +283,10 @@ struct UBuild {
   // TemporalAttention.forward (models/unet3d.py:163-194), folded: x += Wpv * sum_t GN(x) + (T*u + bp)
   void attn(const std::string& name, const AttnW& a, Act& x, const stat_t* stats_x, float* tsum = nullptr, int TS = 0) {
     const int B = up.B, T = x.D, P = x.H * x.W, C = x.C;
+    if (u.attention == ATTN_SOFTMAX) {
+      attn_softmax(name, a, x, stats_x);
+      return;
+    }
     if (tsum) {
       std::vector<float> bias(C, 0.f);
       for (int i = 0; i < C; ++i) bias[i] = (float)T * a.u[i] + a.bp[i];
@@ -300,6 +346,62 @@ struct UBuild {
       b.ops.push_back(std::move(op));
     }
     b.free(y);
+  }
+
+  // softmax attention over the T depth tokens: h = GN(x); q, k, v = qkv(h); o = softmax(q k^T / sqrt(hd)) v per
+  // (position, head); x <- [Wp | I] (o, x) + bp = proj_out(o) + x.  The block output replaces x.
+  void attn_softmax(const std::string& name, const AttnW& a, Act& x, const stat_t* stats_x) {
+    const int B = up.B, T = x.D, P = x.H * x.W, C = x.C, heads = u.desc.num_heads;
+    const double elems = (double)B * T * P;
+    Act h = b.alloc(C, T, x.H, x.W);
+    if (!b.ok) return;
+    {
+      const __half* xp = x.p;
+      __half* hp = h.p;
+      const float *ga = a.norm.gamma, *be = a.norm.beta;
+      const int G = a.norm.G;
+      Op op;
+      op.name = name + ".gn";
+      op.bytes = elems * C * 2.0 * 2.0;
+      op.out = hp;
+      op.out_bytes = (size_t)B * T * P * C * 2;
+      op.run = [=](cudaStream_t st) {
+        launch_gn_apply(xp, hp, stats_x, ga, be, nullptr, 0, nullptr, B, (long long)T * P, C, G, 1e-5f, 2, nullptr, 0,
+                        st);
+      };
+      b.ops.push_back(std::move(op));
+    }
+    Act qkv = b.conv(name + ".qkv", a.qkv, h, nullptr, nullptr, 0);
+    b.free(h);
+    if (!b.ok) return;
+    b.ops.back().bytes = elems * (C + 3.0 * C) * 2.0;
+    Act o = b.alloc(C, T, x.H, x.W);
+    if (!b.ok) return;
+    {
+      TAttnPlan plan;
+      std::string err;
+      if (tattn_plan(plan, qkv.p, o.p, B, T, P, C, heads, err)) {
+        fail(name + ": " + err);
+        b.ok = false;
+        return;
+      }
+      Op op;
+      op.name = name + ".core";
+      op.flops = plan.flops;
+      op.bytes = plan.bytes;
+      op.out = o.p;
+      op.out_bytes = (size_t)B * T * P * C * 2;
+      op.run = [plan](cudaStream_t st) { tattn_launch(plan, st); };
+      b.ops.push_back(std::move(op));
+    }
+    Act y = b.conv(name + ".proj", a.proj, o, &x, nullptr, 0);
+    if (!b.ok) return;
+    b.ops.back().flops = 2.0 * elems * (double)C * C;  // proj_out; the identity half (the residual add) is not counted
+    b.ops.back().bytes = elems * C * 2.0 * 3.0;
+    b.free(qkv);
+    b.free(o);
+    b.free(x);
+    x = y;
   }
 };
 
@@ -377,7 +479,7 @@ static int build_unet_program(UNet& u, UProgram& up) {
       const bool at = !lv.attn.empty();
       float* tsum = nullptr;
       int TS = 0;
-      const bool fz = at && attn_fused(lv.attn[i].C);
+      const bool fz = at && u.attention == ATTN_REFERENCE && attn_fused(lv.attn[i].C);
       Act nxt = ub.res(nm, lv.res[i], cur, nullptr, at ? &cur_stats : nullptr, at ? lv.attn[i].norm.G : 0,
                        fz ? &tsum : nullptr, &TS);
       b.free(cur);
@@ -396,7 +498,7 @@ static int build_unet_program(UNet& u, UProgram& up) {
     float* tsum = nullptr;
     int TS = 0;
     Act nxt = ub.res("mid1", u.mid1, cur, nullptr, &cur_stats, u.mid_attn.norm.G,
-                     attn_fused(u.mid_attn.C) ? &tsum : nullptr, &TS);
+                     (u.attention == ATTN_REFERENCE && attn_fused(u.mid_attn.C)) ? &tsum : nullptr, &TS);
     if (!cur_is_skip) b.free(cur);
     cur = nxt;
     ub.attn("mid.attn", u.mid_attn, cur, cur_stats, tsum, TS);
@@ -415,7 +517,7 @@ static int build_unet_program(UNet& u, UProgram& up) {
       Act nxt;
       float* tsum = nullptr;
       int TS = 0;
-      float** tso = (at && attn_fused(lv.attn[i].C)) ? &tsum : nullptr;
+      float** tso = (at && u.attention == ATTN_REFERENCE && attn_fused(lv.attn[i].C)) ? &tsum : nullptr;
       if (i == 0) {
         Act skip = skips.back();
         skips.pop_back();

@@ -12,9 +12,11 @@ struct ResW {  // ResBlock3D (models/unet3d.py:77-133)
   int cin0 = 0, cin1 = 0, cout = 0;
   int temb_off = 0;  // row offset of this block's time_mlp projection in the concatenated table
 };
-struct AttnW {  // TemporalAttention (models/unet3d.py:136-194), folded
+struct AttnW {  // TemporalAttention (models/unet3d.py:136-194): folded (reference mode) or qkv / proj (softmax mode)
   GNW norm;
   ConvLayer pv;
+  ConvLayer qkv;   // softmax mode: the qkv 1x1 conv, C -> 3C
+  ConvLayer proj;  // softmax mode: dual-source 1x1 conv over (o, x) with weight [Wproj | I_C], bias bproj
   __half* Wt = nullptr;  // [c][co] fp16 transpose of the folded Wp*Wv (fused attn_proj_add path; owned by UNet::ds)
   std::vector<float> u, bp;
   int C = 0;
@@ -48,8 +50,11 @@ struct UProgram {
   int desc_rows = 0;  // rows of one time-embedding projection table (= UNet::proj_rows)
 };
 
+enum { ATTN_REFERENCE = 0, ATTN_SOFTMAX = 1 };  // b2v_unet_set_attention modes
+
 struct UNet {
   b2v_unet_desc desc;
+  int attention = ATTN_REFERENCE;
   WeightMap wm;
   bool finalized = false;
   DeviceStore ds;
@@ -67,6 +72,7 @@ struct UNet {
   long long clock = 0;
 
   int finalize();
+  int set_attention(int mode);  // before finalize; validates every attention level's head_dim for softmax mode
   UProgram* program(int B, int T, int h, int w);
   int forward(const float* x, const long long* t, const float* c, float* eps_out, int B, int T, int h, int w,
               cudaStream_t st);

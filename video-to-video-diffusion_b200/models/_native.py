@@ -51,9 +51,10 @@ class NativeHandle:
         self.version = None
         self.device = None
 
-    def get(self, module, desc, device):
+    def get(self, module, desc, device, attention=None):
+        """attention (U-Net only): the b2v_unet_set_attention mode, part of the cache key; None leaves the default"""
         device = normalize_device(device)
-        ver = _weights_version(module)
+        ver = (_weights_version(module), attention)
         if self.handle is not None and self.version == ver and self.device == device:
             return self.handle
         self.close()
@@ -61,6 +62,8 @@ class NativeHandle:
         h = ctypes.c_void_p()
         with torch.cuda.device(device):
             _lib.check(getattr(L, f"b2v_{self.kind}_create")(ctypes.byref(h), ctypes.byref(desc)), f"{self.kind}_create")
+            if attention is not None:
+                _lib.check(L.b2v_unet_set_attention(h, int(attention)), "unet_set_attention")
             load = getattr(L, f"b2v_{self.kind}_load_weight")
             for key, val in module.state_dict().items():
                 w = val.detach().to("cpu", torch.float32).contiguous()

@@ -53,6 +53,8 @@ class VideoToVideoDiffusion(nn.Module):
                            channel_mult=tuple(config.get("unet_channel_mult", [1, 2, 4, 4])),
                            num_heads=config.get("unet_num_heads", 4),
                            time_embed_dim=config.get("unet_time_embed_dim", 512), use_checkpoint=ckpt)
+        # not a reference key: "softmax" runs checkpoints trained with the corrected attention contraction
+        self.unet.set_attention_mode(config.get("unet_attention", "reference"))
         self.diffusion = GaussianDiffusion(noise_schedule=config.get("noise_schedule", "cosine"),
                                            timesteps=config.get("diffusion_timesteps", 1000),
                                            beta_start=config.get("beta_start", 0.0001),

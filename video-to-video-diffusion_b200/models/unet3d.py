@@ -2,7 +2,7 @@
 parameter names, creation order (so torch's default initialisers draw the same random numbers) and
 `forward(x, t, c)` semantics.  The forward pass itself is one call into libb2v.so (b2v_unet_forward): tcgen05
 implicit-GEMM convolutions, fused GroupNorm/SiLU/time-embedding/residual kernels, the reference's (degenerate)
-temporal attention, all replayed as a CUDA graph.  See csrc/unet.cu and DESIGN.md.
+temporal attention or, opt-in, softmax attention over depth, all replayed as a CUDA graph.  See csrc/unet.cu and DESIGN.md.
 """
 import torch
 import torch.nn as nn
@@ -70,8 +70,32 @@ class Upsample3D(ParamsOnly):
         self.conv = nn.ConvTranspose3d(channels, channels, (3, 4, 4), (1, 2, 2), (1, 1, 1))
 
 
+ATTENTION_MODES = {"reference": 0, "softmax": 1}  # b2v_unet_set_attention codes
+
+
+def softmax_head_dim_error(model_channels, channel_mult, attention_levels, num_heads):
+    """why softmax attention cannot run for this configuration, or None: every attention level and the mid block need
+    head_dim = channels / num_heads to be a multiple of 16 in [16, 128] (the fused attention kernel's tile shapes)"""
+    nl = len(channel_mult)
+    levels = sorted({int(lv) for lv in attention_levels if 0 <= int(lv) < nl} | {nl - 1})
+    for lv in levels:
+        C = model_channels * int(channel_mult[lv])
+        if num_heads < 1 or C % num_heads:
+            return f"{C} channels are not divisible by num_heads = {num_heads}"
+        hd = C // num_heads
+        if hd % 16 or not 16 <= hd <= 128:
+            return (f"head_dim = {C} / {num_heads} = {hd} at {C} channels; softmax attention needs a multiple of 16 "
+                    "in [16, 128]")
+    return None
+
+
 class UNet3D(nn.Module):
-    """eps = UNet3D(...)(x, t, c) with x, c: (B, latent_dim, T, h, w) fp32 CUDA and t: (B,) int64."""
+    """eps = UNet3D(...)(x, t, c) with x, c: (B, latent_dim, T, h, w) fp32 CUDA and t: (B,) int64.
+
+    `attention_mode` selects what TemporalAttention computes: "reference" (default) follows the reference's
+    'bhqk,bhvc->bhqc' contraction exactly (its output does not depend on q, k or the softmax); "softmax" is ordinary
+    attention over the T depth tokens ('bhqk,bhkc->bhqc'), for checkpoints trained with that contraction.  The mode is
+    not stored in the state_dict: set it with `set_attention_mode`."""
 
     def __init__(self, latent_dim=4, model_channels=128, num_res_blocks=2, attention_levels=[1, 2],
                  channel_mult=(1, 2, 4, 4), num_heads=4, time_embed_dim=512, use_checkpoint=False):
@@ -123,6 +147,18 @@ class UNet3D(nn.Module):
         self.conv_out = nn.Sequential(nn.GroupNorm(_groups(ch), ch), nn.SiLU(),
                                       nn.Conv3d(ch, latent_dim, kernel_size=3, padding=1))
         self._native = NativeHandle("unet")
+        self.attention_mode = "reference"
+
+    def set_attention_mode(self, mode):
+        """"reference" | "softmax"; raises ValueError for another mode or a head_dim the softmax kernel cannot run"""
+        if mode not in ATTENTION_MODES:
+            raise ValueError(f"UNet3D: unknown attention mode {mode!r} (expected one of {sorted(ATTENTION_MODES)})")
+        if mode == "softmax":
+            why = softmax_head_dim_error(self.model_channels, self.channel_mult, self.attention_levels, self.num_heads)
+            if why:
+                raise ValueError(f"UNet3D: softmax attention is not supported here: {why}")
+        self.attention_mode = mode
+        return self
 
     # ---- native plumbing
     def _desc(self):
@@ -137,7 +173,7 @@ class UNet3D(nn.Module):
 
     def native(self, device):
         """the b2v_unet handle holding this module's current weights on `device`"""
-        return self._native.get(self, self._desc(), device)
+        return self._native.get(self, self._desc(), device, ATTENTION_MODES[self.attention_mode])
 
     def invalidate_native(self):
         """call after changing weights in a way torch's version counters cannot see (writes through `.data`)"""

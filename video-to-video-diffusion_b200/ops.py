@@ -77,7 +77,8 @@ class Conv:
 
 
 def gn_apply(y, stats, gamma, beta, groups, temb=None, res=None, mode=0, groups_out=0):
-    """y: cl16 (B,D,H,W,C).  mode 0: silu(gn(y)) + temb ; mode 1: silu(gn(y) + res).  Returns (out, stats_out)."""
+    """y: cl16 (B,D,H,W,C).  mode 0: silu(gn(y)) + temb ; mode 1: silu(gn(y) + res) ; mode 2: gn(y).
+    Returns (out, stats_out)."""
     B, D, H, W, C = y.shape
     out = torch.empty_like(y)
     so = torch.zeros((B, groups_out, 2), dtype=torch.int64, device=y.device) if groups_out else None
@@ -100,6 +101,22 @@ def res_attn_tail(y, res, stats_in, gamma2, beta2, groups2, gamma_a, beta_a, gro
         _lib.dptr(out, torch.float16), _lib.dptr(res, torch.float16), _lib.dptr(stats_in, torch.int64), _lib.dptr(gamma2),
         _lib.dptr(beta2), groups2, _lib.dptr(gamma_a), _lib.dptr(beta_a), groups_a, _lib.dptr(wt, torch.float16),
         _lib.dptr(bias), _lib.dptr(sm, torch.int64), _lib.dptr(ws), ws.numel(), B, D, H * W, C, _lib.stream()), "res_attn_tail")
+    return out
+
+
+def temporal_attention(qkv, heads):
+    """softmax attention over depth: qkv cl16 (B,T,H,W,3C) (the qkv 1x1 conv output) -> o cl16 (B,T,H,W,C),
+    o[..., h*hd:(h+1)*hd] = softmax(q k^T / sqrt(hd)) v over the T tokens of each position and head h"""
+    B, T, H, W, C3 = qkv.shape
+    if C3 % 3:
+        raise ValueError(f"temporal_attention: last dim {C3} is not 3C")
+    C = C3 // 3
+    out = torch.empty((B, T, H, W, C), dtype=torch.float16, device=qkv.device)
+    if out.numel() == 0:
+        return out
+    with torch.cuda.device(qkv.device):
+        _lib.check(_lib.lib().b2v_temporal_attention(_lib.dptr(qkv, torch.float16), _lib.dptr(out, torch.float16), B, T,
+                                                     H * W, C, int(heads), _lib.stream()), "temporal_attention")
     return out
 
 
