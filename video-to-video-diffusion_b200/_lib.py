@@ -52,6 +52,10 @@ SIGNATURES = {
     "b2v_unet_forward": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P]),
     "b2v_ddim_sample": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, POINTER(c_int64), c_int, POINTER(c_float),
                                 c_int, c_float, _P, _P, _P]),
+    "b2v_dpmpp_coefficients": (c_int, [POINTER(c_int64), c_int, POINTER(c_float), c_int, c_int, c_int, POINTER(c_float)]),
+    "b2v_dpmpp_sample": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, POINTER(c_int64), c_int, POINTER(c_float),
+                                 c_int, c_int, c_int, _P, _P, _P]),
+    "b2v_dpmpp_update": (c_int, [_P, _P, _P, _P, _P, c_longlong, _P, _P]),
     "b2v_sampler_begin": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, _P]),
     "b2v_ddpm_step": (c_int, [_P, c_int64, POINTER(c_float), _P, _P]),
     "b2v_sampler_end": (c_int, [_P, _P, _P]),

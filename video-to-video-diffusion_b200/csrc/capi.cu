@@ -97,6 +97,17 @@ int b2v_ddim_sample(b2v_unet* u, const float* z_init, const float* cond, float* 
   return u->u.ddim_sample(z_init, cond, z_out, B, T, h, w, (const long long*)timesteps, n, alphas_cumprod, n_train,
                           eta, noise, nan_flag, (cudaStream_t)stream);
 }
+int b2v_dpmpp_coefficients(const int64_t* timesteps, int n, const float* alphas_cumprod, int n_train, int order, int sde,
+                           float* rows) {
+  return dpmpp_coefficients((const long long*)timesteps, n, alphas_cumprod, n_train, order, sde, rows);
+}
+int b2v_dpmpp_sample(b2v_unet* u, const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                     const int64_t* timesteps, int n, const float* alphas_cumprod, int n_train, int order, int sde,
+                     const float* noise, int* nan_flag, void* stream) {
+  if (!u) return fail("dpmpp_sample: null handle");
+  return u->u.dpmpp_sample(z_init, cond, z_out, B, T, h, w, (const long long*)timesteps, n, alphas_cumprod, n_train,
+                           order, sde, noise, nan_flag, (cudaStream_t)stream);
+}
 int b2v_sampler_begin(b2v_unet* u, const float* z_init, const float* cond, int B, int T, int h, int w, void* stream) {
   if (!u) return fail("sampler_begin: null handle");
   return u->u.sampler_begin(z_init, cond, B, T, h, w, (cudaStream_t)stream);
@@ -143,6 +154,16 @@ int b2v_generate(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const floa
                  float* v_out, int B, int T_in, int T_out, int H, int W, int* nan_flag, void* stream) {
   if (!u || !v || !cfg || !v_in || !z_init || !v_out) return fail("generate: null argument");
   if (B < 0 || T_in < 1 || T_out < 1 || H < 4 || W < 4 || H % 4 || W % 4) return fail("generate: bad shape");
+  if (cfg->sampler < 0 || cfg->sampler > 3)
+    return fail("generate: unknown sampler (0 = ddim, 1 = ddpm, 2 = dpmpp_2m, 3 = dpmpp_2m_sde)");
+  if (cfg->sampler >= 2) {  // reject a bad DPM-Solver++ configuration before the encoder is launched
+    if (cfg->sampler == 3 && !cfg->noise) return fail("generate: dpmpp_2m_sde needs the per-step noise draws");
+    if (cfg->n < 1 || cfg->n > 4096) return fail("generate: 1 <= n <= 4096 timesteps");
+    std::vector<float> rows((size_t)cfg->n * 8);
+    if (dpmpp_coefficients((const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod, cfg->n_train, 2,
+                           cfg->sampler == 3, rows.data()))
+      return -1;
+  }
   if (B == 0) return 0;
   if (u->u.desc.latent_dim != v->v.desc.latent_dim) return fail("generate: U-Net / VAE latent_dim mismatch");
   cudaStream_t st = (cudaStream_t)stream;
@@ -183,8 +204,10 @@ int b2v_generate(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const floa
     if (u->u.ddpm_sample(z_init, c, z0, B, T_out, h, w, cfg->ddpm_coef, cfg->n, cfg->noise,
                          (unsigned long long)cfg->seed, st))
       return -1;
-  } else {
-    return fail("generate: unknown sampler (0 = ddim, 1 = ddpm)");
+  } else if (cfg->sampler == 2 || cfg->sampler == 3) {
+    if (u->u.dpmpp_sample(z_init, c, z0, B, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
+                          cfg->n_train, 2, cfg->sampler == 3, cfg->noise, flag + 1, st))
+      return -1;
   }
   launch_guard(z0, (long long)n_z, 1, flag, st);
   if (v->v.decode(z0, v_out, B, T_out, h, w, st)) return -1;
@@ -463,6 +486,14 @@ int b2v_ddim_update(float* z, const float* eps, const float* noise, const float*
   g_launches += 1;
   B2V_CUDA(cudaGetLastError());
   return 0;
+}
+int b2v_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* noise, const float* coef, long long n,
+                     int* nan_flag, void* stream) {
+  if (!z || !x0_prev || !eps || !coef) return fail("dpmpp_update: null argument");
+  if (n <= 0) return 0;
+  launch_dpmpp_update(z, x0_prev, eps, noise, coef, nullptr, n, nan_flag, (cudaStream_t)stream);
+  g_launches += 1;
+  return check_launches("dpmpp_update");
 }
 
 }  // extern "C"

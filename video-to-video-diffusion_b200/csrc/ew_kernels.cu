@@ -742,6 +742,36 @@ __global__ void ddim_update_kernel(float* z, const float* __restrict__ eps, cons
   if (flag && nan_flag) atomicOr(nan_flag, 1);
 }
 
+// DPM-Solver++(2M) update (Lu et al. 2022, data prediction; see b2v_dpmpp_coefficients for the rows), in this fp32
+// order so that a torch eager chain reproduces it bit for bit:
+//   row = {sigma_t, alpha_t, a, b, w0, w1, c, clip}
+//   x0 = clamp(guard((z - sigma_t*e) / alpha_t), +-clip);  D = w1 == 0 ? x0 : w0*x0 + w1*x0_prev
+//   z = guard(a*z + b*D [+ c*noise]);  x0_prev = x0
+// x0_prev is not read when w1 == 0 (it is uninitialised before the first step), noise not when c == 0.
+__global__ void dpmpp_update_kernel(float* z, float* x0_prev, const float* __restrict__ eps,
+                                    const float* __restrict__ noise_imm, const float* __restrict__ coef_table,
+                                    const SamplerCtl* __restrict__ ctl, long long n, int* nan_flag) {
+  pdl_trigger();
+  pdl_wait();
+  const int step = ctl ? ctl->step : 0;
+  const float* c = coef_table + (size_t)step * 8;
+  const float sig = c[0], alp = c[1], a = c[2], b = c[3], w0 = c[4], w1 = c[5], cn = c[6], clip = c[7];
+  const float* noise = cn != 0.f ? (ctl ? ctl_noise(ctl, step, n) : noise_imm) : nullptr;
+  int flag = 0;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const float e = nan_guard(eps[i], &flag);
+    const float zi = z[i];
+    float x0 = nan_guard(__fdiv_rn(__fsub_rn(zi, __fmul_rn(sig, e)), alp), &flag);
+    x0 = fminf(fmaxf(x0, -clip), clip);
+    const float D = (w1 == 0.f) ? x0 : __fadd_rn(__fmul_rn(w0, x0), __fmul_rn(w1, x0_prev[i]));
+    float zn = __fadd_rn(__fmul_rn(a, zi), __fmul_rn(b, D));
+    if (noise) zn = __fadd_rn(zn, __fmul_rn(cn, noise[i]));
+    z[i] = nan_guard(zn, &flag);
+    x0_prev[i] = x0;
+  }
+  if (flag && nan_flag) atomicOr(nan_flag, 1);
+}
+
 // Philox4x32-10 (Salmon et al., SC'11; the counter-based generator behind cuRAND / torch CUDA): counter
 // (c0..c3), key (k0, k1) -> four 32-bit words.  Used for the DDPM ancestral noise when the caller passes none.
 __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
@@ -832,6 +862,12 @@ void launch_ddim_update(float* z, const float* eps, const float* noise, const fl
   int blocks = cdiv(n, 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
   launch_k(ddim_update_kernel, dim3(blocks), dim3(256), 0, st, z, eps, noise, coef_table, ctl, step_imm, n, nan_flag);
+}
+void launch_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* noise, const float* coef_table,
+                         const SamplerCtl* ctl, long long n, int* nan_flag, cudaStream_t st) {
+  int blocks = cdiv(n, 256);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  launch_k(dpmpp_update_kernel, dim3(blocks), dim3(256), 0, st, z, x0_prev, eps, noise, coef_table, ctl, n, nan_flag);
 }
 void launch_ddpm_update(float* z, const float* eps, const float* noise, const float* coef_table, const SamplerCtl* ctl,
                         const Coef8& coef, long long n, cudaStream_t st) {

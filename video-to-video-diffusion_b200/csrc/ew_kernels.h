@@ -43,6 +43,9 @@ void launch_ddim_update(float* z, const float* eps, const float* noise, const fl
                         int step_imm, long long n, int* nan_flag, cudaStream_t st);
 void launch_ddpm_update(float* z, const float* eps, const float* noise, const float* coef_table, const SamplerCtl* ctl,
                         const Coef8& coef, long long n, cudaStream_t st);
+// DPM-Solver++(2M) step: row `step` of coef_table (ctl != null) or coef_table[0..7] with immediate noise (ctl == null)
+void launch_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* noise, const float* coef_table,
+                         const SamplerCtl* ctl, long long n, int* nan_flag, cudaStream_t st);
 void launch_philox_fill(float* out, unsigned long long seed, int step, long long n, cudaStream_t st);
 void launch_guard(float* x, long long n, int mode, int* flag, cudaStream_t st);
 void launch_or_flag(int* dst, const int* src, cudaStream_t st);  // *dst |= *src

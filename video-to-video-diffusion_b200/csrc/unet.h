@@ -35,7 +35,9 @@ struct UProgram {
   Pool pool;
   std::vector<Op> core;
   Program fwd, ddim, ddpm;  // one U-Net evaluation | + DDIM update + advance | + DDPM update + advance
+  Program dpmpp;            // + DPM-Solver++(2M) update + advance
   float *x_in = nullptr, *c_in = nullptr, *eps = nullptr;
+  float* x0_prev = nullptr;  // previous step's data prediction (DPM-Solver++), allocated by the first dpmpp_sample
   long long *t_dev = nullptr, *t_table = nullptr;
   SamplerCtl* ctl = nullptr;  // device loop state of the sampler graphs (step counter, NaN flag, noise source)
   int *step_dev = nullptr, *nan_dev = nullptr;  // = &ctl->step, &ctl->nan_flag
@@ -80,6 +82,10 @@ struct UNet {
   int ddim_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
                   const long long* timesteps, int n, const float* ac, int n_train, float eta, const float* noise,
                   int* nan_flag, cudaStream_t st);
+  // DPM-Solver++(2M) over the timesteps (rows from dpmpp_coefficients); sde: noise = DEVICE [n][numel]
+  int dpmpp_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                   const long long* timesteps, int n, const float* ac, int n_train, int order, int sde,
+                   const float* noise, int* nan_flag, cudaStream_t st);
   int ddpm_step(long long t, const float* coef, const float* noise, cudaStream_t st);
   // loop steps [first, first + count) of an n-step ancestral loop (step s handles timestep n-1-s)
   int ddpm_run(const float* coef, int n, int first, int count, const float* noise, unsigned long long seed,
@@ -90,5 +96,9 @@ struct UNet {
   int sampler_end(float* z_out, cudaStream_t st);
   ~UNet();
 };
+
+// host fp64 coefficient rows of DPM-Solver++(2M) (see b2v_dpmpp_coefficients); no device needed
+int dpmpp_coefficients(const long long* timesteps, int n, const float* ac, int n_train, int order, int sde,
+                       float* rows);
 
 }  // namespace b2v

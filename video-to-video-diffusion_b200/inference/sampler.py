@@ -149,6 +149,87 @@ class DDIMSampler(_Stitching):
                             patch_size, target_patch_size, stride, device)
 
 
+def dpmpp_coefficients(timesteps, alphas_cumprod, order=2, stochastic=False):
+    """the (n, 8) fp32 rows {sigma_t, alpha_t, a, b, w0, w1, c, clip} of a DPM-Solver++(2M) loop over `timesteps`
+    (strictly decreasing), computed in fp64 by b2v_dpmpp_coefficients (host only, no device needed)"""
+    ts = np.ascontiguousarray(timesteps, dtype=np.int64)
+    acp = alphas_cumprod.detach().float().cpu().contiguous()
+    rows = torch.empty((len(ts), 8), dtype=torch.float32)
+    _lib.check(_lib.lib().b2v_dpmpp_coefficients(
+        ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), len(ts), ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)),
+        acp.numel(), int(order), int(bool(stochastic)), ctypes.cast(rows.data_ptr(), ctypes.POINTER(ctypes.c_float))),
+        "dpmpp_coefficients")
+    return rows
+
+
+class DPMSolverSampler(_Stitching):
+    """DPM-Solver++(2M) (Lu et al. 2022), not in the reference: a second-order multistep solver over the same
+    eps-prediction U-Net, one evaluation per step like DDIM, over DDIMSampler's timestep subset (so
+    `num_inference_steps` means the same number of evaluations).  stochastic=True is the 2M SDE form.  With a native
+    UNet3D the whole loop is one call (b2v_dpmpp_sample); any other callable model runs a Python loop over the same
+    update kernel.  RNG order: z = randn(shape), then (SDE only) one randn_like per step."""
+
+    def __init__(self, diffusion, model):
+        self.diffusion, self.model, self.timesteps = diffusion, model, diffusion.timesteps
+
+    def _get_timesteps(self, num_inference_steps):
+        return DDIMSampler._get_timesteps(self, num_inference_steps)
+
+    @torch.no_grad()
+    def sample(self, shape, conditioning, num_inference_steps, device, order=2, stochastic=False, progress=True):
+        if order not in (1, 2):
+            raise ValueError(f"DPMSolverSampler: order must be 1 or 2, got {order}")
+        ts = np.ascontiguousarray(self._get_timesteps(num_inference_steps), dtype=np.int64)
+        n = len(ts)
+        acp = self.diffusion.alphas_cumprod.detach().float().cpu().contiguous()
+        native = _is_native(self.model)
+        if native:
+            shape, dev = check_sampler_args(self.model, shape, conditioning, device)  # ValueError before any C call
+        else:
+            dev = torch.device(device)
+        z = torch.randn(shape, device=dev)
+        cond = conditioning.detach().to(dev, torch.float32).contiguous()
+        if z.numel() == 0:
+            return z
+        noise = torch.stack([torch.randn_like(z) for _ in range(n)]).contiguous() if stochastic else None
+        if not native:
+            return self._sample_generic(z, cond, ts, dpmpp_coefficients(ts, acp, order, stochastic).to(dev), noise)
+        B, _, T, h, w = shape
+        out = torch.empty_like(z)
+        flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().b2v_dpmpp_sample(
+                self.model.native(dev), _lib.dptr(z), _lib.dptr(cond), _lib.dptr(out), B, T, h, w,
+                ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), n,
+                ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)), acp.numel(), int(order), int(stochastic),
+                _lib.dptr(noise), _lib.dptr(flag, torch.int32), _lib.stream()), "dpmpp_sample")
+        self.last_nan_flag = flag  # device tensor; .item() it to learn whether a NaN/Inf guard fired
+        return out
+
+    def _sample_generic(self, z, cond, ts, rows, noise):
+        """any callable model(z, t, c): Python loop, the update kernel per step (in place on z)"""
+        dev = z.device
+        x0_prev = torch.empty_like(z)
+        flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        for i, t_idx in enumerate(ts):
+            t = torch.full((z.shape[0],), int(t_idx), device=dev, dtype=torch.long)
+            eps = self.model(z, t, cond).float().contiguous()
+            flag |= ops.dpmpp_update(z, x0_prev, eps, rows[i].contiguous(), None if noise is None else noise[i])
+        self.last_nan_flag = flag
+        return z
+
+    @torch.no_grad()
+    def sample_with_stitching(self, v_thick_full, vae, num_inference_steps: int = 20,
+                              patch_size: Tuple[int, int, int] = (8, 192, 192),
+                              target_patch_size: Tuple[int, int, int] = (48, 192, 192),
+                              stride: Tuple[int, int, int] = (4, 96, 96), device="cuda", order=2, stochastic=False,
+                              progress=True):
+        return self._stitch(v_thick_full, vae,
+                            lambda s, c: self.sample(s, c, num_inference_steps, device, order=order,
+                                                     stochastic=stochastic, progress=False),
+                            patch_size, target_patch_size, stride, device)
+
+
 class EDMSampler:
     def __init__(self, diffusion, model):
         raise NotImplementedError("EDM sampler not yet implemented")  # same as the reference (:482-493)

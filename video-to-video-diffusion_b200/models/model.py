@@ -1,7 +1,7 @@
 """Mirror of the reference `models/model.py` facade: `VideoToVideoDiffusion(config)` resolves the config the way
 the reference does (including reading the U-Net keys from the top level of the dict only), exposes `.vae`, `.unet`,
 `.diffusion` under the same names so reference checkpoints load, and `generate()` runs
-encode -> depth upsample -> DDIM/DDPM -> decode entirely on libb2v.so.  Training (`forward`, `save_checkpoint`)
+encode -> depth upsample -> DDIM/DDPM (or DPM-Solver++(2M), not in the reference) -> decode entirely on libb2v.so.  Training (`forward`, `save_checkpoint`)
 is out of scope of this package.
 """
 import ctypes
@@ -76,8 +76,9 @@ class VideoToVideoDiffusion(nn.Module):
     @torch.no_grad()
     def generate(self, v_in, sampler, num_inference_steps=20, guidance_scale=1.0, target_depth=None):
         """thick slices (B,C,T_in,H,W) -> thin slices (B,C,T_out,H,W), fp32, tanh-bounded.  `guidance_scale` is
-        accepted and ignored, exactly like the reference."""
-        if sampler not in ("ddpm", "ddim"):
+        accepted and ignored, exactly like the reference.  Besides the reference's "ddim" / "ddpm", `sampler` may be
+        "dpmpp_2m" or "dpmpp_2m_sde" (DPM-Solver++(2M), ODE / SDE: num_inference_steps as for DDIM)."""
+        if sampler not in ("ddpm", "ddim", "dpmpp_2m", "dpmpp_2m_sde"):
             raise ValueError(f"Unknown sampler: {sampler}")
         device = v_in.device
         B, C, T_in, H, W = v_in.shape
@@ -95,20 +96,25 @@ class VideoToVideoDiffusion(nn.Module):
         if sampler == "ddpm" and n * n_lat * 4 > ddpm_noise_budget_bytes():
             return self._generate_staged(v_in, shape, target_depth)  # per-step noise does not fit: chunked loop
         # RNG order of the reference: a discarded randn(latent_shape) (models/model.py:303), the sampler's initial
-        # draw, then (DDPM) one randn_like per step
+        # draw, then (DDPM, DPM-Solver++ SDE) one randn_like per step
         torch.randn(shape, device=device)
         z_init = torch.randn(shape, device=device)
         cfg = _lib.SamplerCfg()
         keep = []  # host tables must outlive the call
-        if sampler == "ddim":
+        if sampler != "ddpm":
             from ..inference.sampler import DDIMSampler
             ts = np.ascontiguousarray(DDIMSampler(self.diffusion, self.unet)._get_timesteps(num_inference_steps),
                                       dtype=np.int64)
             acp = self.diffusion.alphas_cumprod.detach().float().cpu().contiguous()
             keep += [ts, acp]
-            cfg.sampler, cfg.n, cfg.n_train, cfg.eta = 0, len(ts), acp.numel(), 0.0
+            code = {"ddim": 0, "dpmpp_2m": 2, "dpmpp_2m_sde": 3}[sampler]
+            cfg.sampler, cfg.n, cfg.n_train, cfg.eta = code, len(ts), acp.numel(), 0.0
             cfg.timesteps = ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
             cfg.alphas_cumprod = ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float))
+            if sampler == "dpmpp_2m_sde":
+                noise = torch.stack([torch.randn_like(z_init) for _ in range(len(ts))]).contiguous()
+                keep.append(noise)
+                cfg.noise = noise.data_ptr()
         else:
             rows = self.diffusion.ddpm_coefficients()
             noise = torch.empty((n,) + shape, dtype=torch.float32, device=device)

@@ -136,6 +136,16 @@ def ddim_update(z, eps, coef, noise=None):
     return flag
 
 
+def dpmpp_update(z, x0_prev, eps, coef, noise=None):
+    """in-place DPM-Solver++(2M) step on z and x0_prev (fp32); coef: device fp32[8], one b2v_dpmpp_coefficients row;
+    noise: this step's N(0,1) draw (read when coef[6] != 0).  Returns the NaN flag tensor."""
+    flag = torch.zeros(1, dtype=torch.int32, device=z.device)
+    _lib.check(_lib.lib().b2v_dpmpp_update(_lib.dptr(z), _lib.dptr(x0_prev), _lib.dptr(eps), _lib.dptr(noise),
+                                           _lib.dptr(coef), z.numel(), _lib.dptr(flag, torch.int32), _lib.stream()),
+               "dpmpp_update")
+    return flag
+
+
 def ddpm_update(z, eps, noise, coef_row):
     """in-place DDPM ancestral update of z (fp32); coef_row: 8 host floats (GaussianDiffusion.ddpm_coefficients()[t])"""
     coef = (ctypes.c_float * 8)(*[float(v) for v in coef_row])
