@@ -99,6 +99,29 @@ def test_ddim_loop_equals_oracle_loop_on_gpu(cuda_dev):
         assert rel_l2(got, ref) < 5e-2, (eta, rel_l2(got, ref))
 
 
+@pytest.mark.parametrize("eta", [0.0, 0.5])
+def test_ddim_whole_loop_equals_stepwise_loop(cuda_dev, eta):
+    """b2v_ddim_sample is bitwise the step-wise loop (native forward + ops.ddim_update per step, same draws in the
+    same order: z, then one randn_like per step when eta > 0)"""
+    import numpy as np
+    from v2v_b200.inference import DDIMSampler
+    from v2v_b200.models import GaussianDiffusion
+    m = tiny_unet(0).to(cuda_dev)
+    diff = GaussianDiffusion("cosine", 1000).to(cuda_dev)
+    cond = golden("ddim_tiny.pt")["cond"].to(cuda_dev)
+    shape = (1, 4, 4, 8, 8)
+    torch.manual_seed(7)
+    whole = DDIMSampler(diff, m).sample(shape, cond, 5, cuda_dev, eta=eta, progress=False)
+    smp = DDIMSampler(diff, m)
+    ts = np.ascontiguousarray(smp._get_timesteps(5), dtype=np.int64)
+    acp = diff.alphas_cumprod.detach().float().cpu().contiguous()
+    torch.manual_seed(7)
+    z = torch.randn(shape, device=cuda_dev)
+    with torch.no_grad():
+        stepwise = smp._sample_generic(z, cond, ts, acp, eta)
+    assert torch.equal(whole, stepwise)
+
+
 def test_ddim_generic_model_path(cuda_dev):
     """DDIMSampler accepts any callable model (as the reference does); the update still runs on our kernel"""
     from v2v_b200.inference import DDIMSampler

@@ -243,7 +243,7 @@ int b2v_eps_mse(const float* eps_pred, const float* noise, const float* mask, fl
 int b2v_unet_profile(b2v_unet* u, int iters, char* buf, size_t cap, void* stream) {
   if (!u) return fail("unet_profile: null handle");
   if (!u->u.last) return fail("unet_profile: run a forward first");
-  u->u.last->temb = TembSource{u->u.last->proj, u->u.last->desc_rows, nullptr, 0};
+  u->u.forward_temb(*u->u.last);
   std::string js;
   if (u->u.last->fwd.profile(iters, (cudaStream_t)stream, js)) return -1;
   return write_json(js, buf, cap);
@@ -286,7 +286,7 @@ int b2v_vae_profile(b2v_vae* v, int which, int iters, char* buf, size_t cap, voi
 static Program* debug_prog(void* obj, int prog) {
   if (prog == 0) {
     UNet& u = ((b2v_unet*)obj)->u;
-    if (u.last) u.last->temb = TembSource{u.last->proj, u.last->desc_rows, nullptr, 0};
+    if (u.last) u.forward_temb(*u.last);
     return u.last ? &u.last->fwd : nullptr;
   }
   VAE& v = ((b2v_vae*)obj)->v;
@@ -482,7 +482,7 @@ int b2v_ddpm_update(float* z, const float* eps, const float* noise, const float*
 }
 int b2v_ddim_update(float* z, const float* eps, const float* noise, const float* coef, long long n, int* nan_flag,
                     void* stream) {
-  launch_ddim_update(z, eps, noise, coef, nullptr, 0, n, nan_flag, (cudaStream_t)stream);
+  launch_ddim_update(z, eps, noise, coef, nullptr, n, nan_flag, (cudaStream_t)stream);
   g_launches += 1;
   B2V_CUDA(cudaGetLastError());
   return 0;

@@ -633,10 +633,9 @@ void launch_attn_proj_add(__half* x, const float* tsum, int TS, const stat_t* st
 // Time embedding (reference models/unet3d.py:18-48 and the per-block time_mlp :88-91,123-125).
 //   temb_mlp : sinusoid(t) -> Linear(dim,td) -> SiLU -> Linear(td,td); stores SiLU(temb) (what every block consumes)
 //   temb_proj: all ResBlock projections at once: out[b][row] = W[row,:].silu_temb[b,:] + bias[row]
-// t comes from t_ptr[b], or from t_table[*step_ptr] when a sampler graph is replayed.
+// t comes from t_ptr[b]: one block per sample (forward) or per loop step (the all-steps table of a sampler loop).
 // ------------------------------------------------------------------------------------------------
-__global__ void temb_mlp_kernel(const long long* __restrict__ t_ptr, const long long* __restrict__ t_table,
-                                const int* __restrict__ step_ptr, const float* __restrict__ freqs,
+__global__ void temb_mlp_kernel(const long long* __restrict__ t_ptr, const float* __restrict__ freqs,
                                 const float* __restrict__ W1, const float* __restrict__ b1,
                                 const float* __restrict__ W2, const float* __restrict__ b2, float* silu_temb,
                                 int dim, int td) {
@@ -646,7 +645,7 @@ __global__ void temb_mlp_kernel(const long long* __restrict__ t_ptr, const long 
   float* emb = sm;
   float* h1 = sm + dim;
   const int b = blockIdx.x;
-  const long long t = t_table ? t_table[*step_ptr] : t_ptr[b];
+  const long long t = t_ptr[b];
   const int half = dim / 2;
   for (int i = threadIdx.x; i < half; i += blockDim.x) {
     const float a = (float)t * freqs[i];
@@ -684,11 +683,11 @@ __global__ void temb_proj_kernel(const float* __restrict__ W, const float* __res
   }
 }
 
-void launch_temb(const long long* t_ptr, const long long* t_table, const int* step_ptr, const float* freqs,
-                 const float* W1, const float* b1, const float* W2, const float* b2, float* silu_temb,
-                 const float* Wp, const float* bp, float* proj, int rows, int dim, int td, int B, cudaStream_t st) {
-  launch_k(temb_mlp_kernel, dim3(B), dim3(512), (dim + td) * sizeof(float), st, t_ptr, t_table, step_ptr, freqs, W1, b1, W2, b2,
-                                                              silu_temb, dim, td);
+void launch_temb(const long long* t_ptr, const float* freqs, const float* W1, const float* b1, const float* W2,
+                 const float* b2, float* silu_temb, const float* Wp, const float* bp, float* proj, int rows, int dim,
+                 int td, int B, cudaStream_t st) {
+  launch_k(temb_mlp_kernel, dim3(B), dim3(512), (dim + td) * sizeof(float), st, t_ptr, freqs, W1, b1, W2, b2, silu_temb,
+           dim, td);
   launch_k(temb_proj_kernel, dim3(cdiv((long long)rows * 32, 256)), dim3(256), 0, st, Wp, bp, silu_temb, proj, rows, td, B);
 }
 
@@ -722,10 +721,10 @@ __device__ __forceinline__ const float* ctl_noise(const SamplerCtl* ctl, int ste
 
 __global__ void ddim_update_kernel(float* z, const float* __restrict__ eps, const float* __restrict__ noise_imm,
                                    const float* __restrict__ coef_table, const SamplerCtl* __restrict__ ctl,
-                                   int step_imm, long long n, int* nan_flag) {
+                                   long long n, int* nan_flag) {
   pdl_trigger();
   pdl_wait();
-  const int step = ctl ? ctl->step : step_imm;
+  const int step = ctl ? ctl->step : 0;
   const float* noise = ctl ? ctl_noise(ctl, step, n) : noise_imm;
   const float* c = coef_table + (size_t)step * 8;
   const float c1 = c[0], c2 = c[1], c3 = c[2], c4 = c[3], sigma = c[4];
@@ -858,10 +857,10 @@ __global__ void advance_step_kernel(SamplerCtl* ctl) {
 }
 
 void launch_ddim_update(float* z, const float* eps, const float* noise, const float* coef_table, const SamplerCtl* ctl,
-                        int step_imm, long long n, int* nan_flag, cudaStream_t st) {
+                        long long n, int* nan_flag, cudaStream_t st) {
   int blocks = cdiv(n, 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
-  launch_k(ddim_update_kernel, dim3(blocks), dim3(256), 0, st, z, eps, noise, coef_table, ctl, step_imm, n, nan_flag);
+  launch_k(ddim_update_kernel, dim3(blocks), dim3(256), 0, st, z, eps, noise, coef_table, ctl, n, nan_flag);
 }
 void launch_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* noise, const float* coef_table,
                          const SamplerCtl* ctl, long long n, int* nan_flag, cudaStream_t st) {
@@ -990,17 +989,16 @@ void launch_zero(float* p, long long n, cudaStream_t st) {
 }
 void launch_advance_step(SamplerCtl* ctl, cudaStream_t st) { launch_k(advance_step_kernel, dim3(1), dim3(1), 0, st, ctl); }
 
-// t_dev[b] = t_table[*step] (sampler graphs) or an immediate value (step-wise DDPM)
-__global__ void set_t_kernel(long long* t_dev, const long long* __restrict__ t_table, const int* __restrict__ step,
-                             long long imm, int B) {
+// t_dev[b] = t for every sample (step-wise DDPM)
+__global__ void set_t_kernel(long long* t_dev, long long t, int B) {
   pdl_trigger();
   pdl_wait();
   const int b = threadIdx.x;
-  if (b < B) t_dev[b] = t_table ? t_table[*step] : imm;
+  if (b < B) t_dev[b] = t;
 }
-void launch_set_t(long long* t_dev, const long long* t_table, const int* step, long long imm, int B, cudaStream_t st) {
+void launch_set_t(long long* t_dev, long long t, int B, cudaStream_t st) {
   const int threads = B < 64 ? 64 : B;
-  launch_k(set_t_kernel, dim3(1), dim3(threads), 0, st, t_dev, t_table, step, imm, B);
+  launch_k(set_t_kernel, dim3(1), dim3(threads), 0, st, t_dev, t, B);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -23,12 +23,12 @@ void launch_attn_proj_add(__half* x, const float* tsum, int TS, const stat_t* st
                           const float* beta, const __half* Wt, const float* bias, __half* g_ws, int B, int T, int P,
                           int C, int G, float eps, cudaStream_t st);
 void launch_add_bcast_t(__half* x, const __half* y, int B, int T, int P, int C, cudaStream_t st);
-void launch_temb(const long long* t_ptr, const long long* t_table, const int* step_ptr, const float* freqs,
-                 const float* W1, const float* b1, const float* W2, const float* b2, float* silu_temb,
-                 const float* Wp, const float* bp, float* proj, int rows, int dim, int td, int B, cudaStream_t st);
+void launch_temb(const long long* t_ptr, const float* freqs, const float* W1, const float* b1, const float* W2,
+                 const float* b2, float* silu_temb, const float* Wp, const float* bp, float* proj, int rows, int dim,
+                 int td, int B, cudaStream_t st);
 // device-resident loop state of a sampler graph (one per U-Net program)
 struct SamplerCtl {
-  int step;                 // loop index: selects the coefficient / timestep / time-embedding row; advanced by the graph
+  int step;                 // loop index: selects the coefficient / noise / time-embedding row; advanced by the graph
   int nan_flag;             // set when one of the reference's NaN/Inf guards fired
   int noise_first;          // loop index of row 0 of `noise`
   int pad;
@@ -38,9 +38,9 @@ struct SamplerCtl {
 struct Coef8 {
   float v[8];
 };
-// ctl != null: step / noise come from the control block (sampler graphs); else step_imm / noise are immediate
+// ctl != null: step / noise come from the control block (sampler graphs); else row 0 of coef_table, immediate noise
 void launch_ddim_update(float* z, const float* eps, const float* noise, const float* coef_table, const SamplerCtl* ctl,
-                        int step_imm, long long n, int* nan_flag, cudaStream_t st);
+                        long long n, int* nan_flag, cudaStream_t st);
 void launch_ddpm_update(float* z, const float* eps, const float* noise, const float* coef_table, const SamplerCtl* ctl,
                         const Coef8& coef, long long n, cudaStream_t st);
 // DPM-Solver++(2M) step: row `step` of coef_table (ctl != null) or coef_table[0..7] with immediate noise (ctl == null)
@@ -57,7 +57,7 @@ void launch_eps_mse(const float* pred, const float* noise, const float* mask, in
 void ew_set_round_bf16(int on);
 void launch_advance_step(SamplerCtl* ctl, cudaStream_t st);
 void launch_zero(float* p, long long n, cudaStream_t st);
-void launch_set_t(long long* t_dev, const long long* t_table, const int* step, long long imm, int B, cudaStream_t st);
+void launch_set_t(long long* t_dev, long long t, int B, cudaStream_t st);
 void launch_pack_unet_in(const float* z, const float* c, __half* out, int B, int L, int D, int H, int W,
                          cudaStream_t st);
 void launch_pack_vae_dec_in(const float* z, const float* Wpq, const float* bpq, float scaling, __half* out, int B,

@@ -405,6 +405,43 @@ struct UBuild {
   }
 };
 
+// the last op of sampler `kind`'s loop program: its update, which reads the coefficient row and the noise through
+// the device control block, then the step advance
+static Op loop_update_op(UProgram& up, int kind) {
+  float* z = up.x_in;
+  const float* e = up.eps;
+  const float* ct = up.coef_table;
+  SamplerCtl* ctl = up.ctl;
+  int* nf = up.nan_dev;
+  const long long numel = up.numel;
+  UProgram* upp = &up;  // x0_prev is allocated by the first dpmpp_sample (before its graph is captured): read at launch
+  Op op;
+  op.launches = 2;
+  switch (kind) {
+    case SAMPLER_DDIM:
+      op.name = "ddim_update";
+      op.bytes = (double)numel * 12.0;
+      op.run = [=](cudaStream_t st) { launch_ddim_update(z, e, nullptr, ct, ctl, numel, nf, st); };
+      break;
+    case SAMPLER_DDPM:
+      op.name = "ddpm_update";
+      op.bytes = (double)numel * 16.0;
+      op.run = [=](cudaStream_t st) { launch_ddpm_update(z, e, nullptr, ct, ctl, Coef8{}, numel, st); };
+      break;
+    case SAMPLER_DPMPP:
+      op.name = "dpmpp_update";
+      op.bytes = (double)numel * 20.0;  // z, eps, x0_prev read; z, x0_prev written (+4 B noise in the SDE form)
+      op.run = [=](cudaStream_t st) { launch_dpmpp_update(z, upp->x0_prev, e, nullptr, ct, ctl, numel, nf, st); };
+      break;
+  }
+  const auto update = std::move(op.run);
+  op.run = [=](cudaStream_t st) {
+    update(st);
+    launch_advance_step(ctl, st);
+  };
+  return op;
+}
+
 static int build_unet_program(UNet& u, UProgram& up) {
   const b2v_unet_desc& d = u.desc;
   const int B = up.B, T = up.T, h = up.h, w = up.w, L = d.latent_dim, NL = d.num_levels;
@@ -412,7 +449,6 @@ static int build_unet_program(UNet& u, UProgram& up) {
     if ((h >> l) & 1 || (w >> l) & 1) return fail("latent H, W must be divisible by 2^(levels-1)");
   const long long numel = (long long)B * L * T * h * w;
   up.numel = numel;
-  up.desc_rows = u.proj_rows;
   up.x_in = (float*)up.ds.alloc(numel * 4);
   up.c_in = (float*)up.ds.alloc(numel * 4);
   up.eps = (float*)up.ds.alloc(numel * 4);
@@ -451,7 +487,7 @@ static int build_unet_program(UNet& u, UProgram& up) {
     op.launches = 2;
     op.bytes = ((double)rows * td + (double)td * td + (double)td * dim) * 4.0;
     op.run = [=](cudaStream_t st) {
-      launch_temb(tp, nullptr, nullptr, fr, W1, B1, W2, B2, st_, Wp, Bp, pj, rows, dim, td, B, st);
+      launch_temb(tp, fr, W1, B1, W2, B2, st_, Wp, Bp, pj, rows, dim, td, B, st);
     };
     b.ops.push_back(std::move(op));
   }
@@ -558,53 +594,12 @@ static int build_unet_program(UNet& u, UProgram& up) {
   if (!b.ok) return -1;
 
   up.fwd.ops = up.core;
-  // sampler steps: core (the time embedding of every step is computed once per sample() call: see temb_tables), the
-  // scheduler update reading its coefficient row / noise through the device control block, advance
-  for (auto& o : up.core)
-    if (o.name != "time_embed") {
-      up.ddim.ops.push_back(o);
-      up.ddpm.ops.push_back(o);
-      up.dpmpp.ops.push_back(o);
-    }
-  {
-    float* z = up.x_in;
-    const float* e = up.eps;
-    const float* ct = up.coef_table;
-    SamplerCtl* ctl = up.ctl;
-    int* nf = up.nan_dev;
-    Op op;
-    op.name = "ddim_update";
-    op.launches = 2;
-    op.bytes = (double)numel * 12.0;
-    op.run = [=](cudaStream_t st) {
-      launch_ddim_update(z, e, nullptr, ct, ctl, 0, numel, nf, st);
-      launch_advance_step(ctl, st);
-    };
-    up.ddim.ops.push_back(op);
-    op.name = "ddpm_update";
-    op.bytes = (double)numel * 16.0;
-    op.run = [=](cudaStream_t st) {
-      launch_ddpm_update(z, e, nullptr, ct, ctl, Coef8{}, numel, st);
-      launch_advance_step(ctl, st);
-    };
-    up.ddpm.ops.push_back(std::move(op));
-  }
-  {  // x0_prev is allocated by the first dpmpp_sample (before this graph is captured), so it is read at launch time
-    float* z = up.x_in;
-    const float* e = up.eps;
-    const float* ct = up.coef_table;
-    SamplerCtl* ctl = up.ctl;
-    int* nf = up.nan_dev;
-    UProgram* upp = &up;
-    Op op;
-    op.name = "dpmpp_update";
-    op.launches = 2;
-    op.bytes = (double)numel * 20.0;  // z, eps, x0_prev read; z, x0_prev written (+4 B noise in the SDE form)
-    op.run = [=](cudaStream_t st) {
-      launch_dpmpp_update(z, upp->x0_prev, e, nullptr, ct, ctl, numel, nf, st);
-      launch_advance_step(ctl, st);
-    };
-    up.dpmpp.ops.push_back(std::move(op));
+  // sampler loop steps: core without time_embed (the time embedding of every step is computed once per loop: see
+  // temb_tables), then the sampler's update and advance
+  for (int k = 0; k < SAMPLER_KINDS; ++k) {
+    for (auto& o : up.core)
+      if (o.name != "time_embed") up.loop[k].ops.push_back(o);
+    up.loop[k].ops.push_back(loop_update_op(up, k));
   }
   return 0;
 }
@@ -647,7 +642,7 @@ int UNet::forward(const float* x, const long long* t, const float* c, float* eps
   B2V_CUDA(cudaMemcpyAsync(up->x_in, x, bytes, cudaMemcpyDeviceToDevice, st));
   B2V_CUDA(cudaMemcpyAsync(up->c_in, c, bytes, cudaMemcpyDeviceToDevice, st));
   B2V_CUDA(cudaMemcpyAsync(up->t_dev, t, sizeof(long long) * B, cudaMemcpyDeviceToDevice, st));
-  up->temb = TembSource{up->proj, proj_rows, nullptr, 0};
+  forward_temb(*up);
   if (up->fwd.run(st)) return -1;
   B2V_CUDA(cudaMemcpyAsync(eps_out, up->eps, bytes, cudaMemcpyDeviceToDevice, st));
   return 0;
@@ -666,45 +661,65 @@ int UNet::sampler_begin(const float* z_init, const float* cond, int B, int T, in
 }
 
 // time embedding + all ResBlock projections for every loop step at once ([n][rows] table, one launch pair)
-int UNet::temb_tables(UProgram* up, int n, cudaStream_t st) {
+static int temb_tables(const UNet& u, UProgram* up, int n, cudaStream_t st) {
   if (up->all_cap < n) {
     B2V_CUDA(cudaStreamSynchronize(st));  // the old tables may be in use by queued work
     if (up->silu_all) up->ds.release(up->silu_all);
     if (up->proj_all) up->ds.release(up->proj_all);
     up->all_cap = 0;
-    up->silu_all = (float*)up->ds.alloc((size_t)n * desc.time_embed_dim * sizeof(float));
-    up->proj_all = (float*)up->ds.alloc((size_t)n * proj_rows * sizeof(float));
+    up->silu_all = (float*)up->ds.alloc((size_t)n * u.desc.time_embed_dim * sizeof(float));
+    up->proj_all = (float*)up->ds.alloc((size_t)n * u.proj_rows * sizeof(float));
     if (!up->silu_all || !up->proj_all) return fail("out of device memory (time-embedding table)");
     up->all_cap = n;
-    for (Program* pr : {&up->ddim, &up->ddpm, &up->dpmpp})
-      if (pr->exec) {  // the captured graphs hold the old table pointer
-        cudaGraphExecDestroy(pr->exec);
-        pr->exec = nullptr;
+    for (Program& pr : up->loop)
+      if (pr.exec) {  // the captured graphs hold the old table pointer
+        cudaGraphExecDestroy(pr.exec);
+        pr.exec = nullptr;
       }
   }
-  launch_temb(up->t_table, nullptr, nullptr, freqs, W1, B1, W2, B2, up->silu_all, Wproj, Bproj, up->proj_all, proj_rows,
-              desc.model_channels, desc.time_embed_dim, n, st);
+  launch_temb(up->t_table, u.freqs, u.W1, u.B1, u.W2, u.B2, up->silu_all, u.Wproj, u.Bproj, up->proj_all, u.proj_rows,
+              u.desc.model_channels, u.desc.time_embed_dim, n, st);
   g_launches += 2;
-  up->temb = TembSource{up->proj_all, 0, up->step_dev, proj_rows};
   return 0;
 }
 
-// coefficient table in the reference's fp32 operation order (inference/sampler.py:295-325)
-int UNet::ddim_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
-                      const long long* timesteps, int n, const float* ac, int n_train, float eta, const float* noise,
-                      int* nan_flag, cudaStream_t st) {
-  if (n < 1 || n > 4096) return fail("ddim_sample: 1 <= n <= 4096 timesteps");
-  if (eta > 0.f && !noise) return fail("ddim_sample: eta > 0 needs the per-step noise draws");
-  if (!timesteps || !ac) return fail("ddim_sample: null schedule");
-  if (sampler_begin(z_init, cond, B, T, h, w, st)) return -1;
-  UProgram* up = active;
-  std::vector<float> coef((size_t)n * 8, 0.f);
-  std::vector<long long> ts(timesteps, timesteps + n);
-  for (int i = 0; i < n; ++i) {
+// the loop driver shared by the samplers.  loop_tables: upload a loop's timesteps and [n][8] coefficient rows (loop
+// order) and build its time embedding.
+static int loop_tables(const UNet& u, UProgram* up, const std::vector<long long>& ts, const std::vector<float>& rows,
+                       cudaStream_t st) {
+  const int n = (int)ts.size();
+  // pageable-host copies are staged by the runtime before returning, so the vectors may go out of scope
+  B2V_CUDA(cudaMemcpyAsync(up->t_table, ts.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, st));
+  B2V_CUDA(cudaMemcpyAsync(up->coef_table, rows.data(), sizeof(float) * 8 * n, cudaMemcpyHostToDevice, st));
+  return temb_tables(u, up, n, st);
+}
+
+// loop_replay: set the noise source (the caller's [rows][numel] draws whose row 0 is loop step `first`, or null: no
+// noise / the Philox seed) and replay loop[kind] `count` times.
+static int loop_replay(const UNet& u, UProgram* up, int kind, int first, int count, const float* noise,
+                       unsigned long long seed, cudaStream_t st) {
+  SamplerCtl c{};  // step / nan_flag are owned by the device (offsetof: the first two ints stay untouched)
+  c.noise_first = first;
+  c.noise = noise;
+  c.seed = seed;
+  const size_t off = offsetof(SamplerCtl, noise_first);
+  B2V_CUDA(cudaMemcpyAsync((char*)up->ctl + off, (const char*)&c + off, sizeof(SamplerCtl) - off,
+                           cudaMemcpyHostToDevice, st));
+  up->temb = TembSource{up->proj_all, 0, up->step_dev, u.proj_rows};
+  for (int i = 0; i < count; ++i)
+    if (up->loop[kind].run(st)) return -1;
+  return 0;
+}
+
+// DDIM rows {c1, c2, c3, c4, sigma, 0, 0, 0} into zeroed `rows`, in the reference's fp32 operation order
+// (inference/sampler.py:295-325)
+static int ddim_coefficients(const long long* ts, int n, const float* ac, int n_train, float eta, float* rows) {
+  for (int i = 0; i < n; ++i)
     if (ts[i] < 0 || ts[i] >= n_train) return fail("ddim_sample: timestep out of range");
+  for (int i = 0; i < n; ++i) {
     const float a_t = ac[ts[i]];
     const float a_prev = (i < n - 1) ? ac[ts[i + 1]] : 1.0f;
-    float* c = &coef[(size_t)i * 8];
+    float* c = rows + (size_t)i * 8;
     c[0] = sqrtf(1.0f - a_t + 1e-8f);
     c[1] = sqrtf(a_t + 1e-8f) + 1e-8f;
     c[2] = sqrtf(a_prev + 1e-8f);
@@ -712,17 +727,22 @@ int UNet::ddim_sample(const float* z_init, const float* cond, float* z_out, int 
     if (eta > 0.f)
       c[4] = eta * sqrtf((1.0f - a_prev + 1e-8f) / (1.0f - a_t + 1e-8f) * (1.0f - a_t / (a_prev + 1e-8f)));
   }
-  // pageable-host copies are staged by the runtime before returning, so the vectors may go out of scope
-  B2V_CUDA(cudaMemcpyAsync(up->t_table, ts.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, st));
-  B2V_CUDA(cudaMemcpyAsync(up->coef_table, coef.data(), sizeof(float) * 8 * n, cudaMemcpyHostToDevice, st));
-  if (eta > 0.f) {  // the stochastic variant reads step i's draw from row i of the caller's buffer
-    SamplerCtl c{};
-    c.noise = noise;
-    B2V_CUDA(cudaMemcpyAsync(up->ctl, &c, sizeof c, cudaMemcpyHostToDevice, st));
-  }
-  if (temb_tables(up, n, st)) return -1;
-  for (int i = 0; i < n; ++i)
-    if (up->ddim.run(st)) return -1;
+  return 0;
+}
+
+int UNet::ddim_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                      const long long* timesteps, int n, const float* ac, int n_train, float eta, const float* noise,
+                      int* nan_flag, cudaStream_t st) {
+  if (n < 1 || n > 4096) return fail("ddim_sample: 1 <= n <= 4096 timesteps");
+  if (eta > 0.f && !noise) return fail("ddim_sample: eta > 0 needs the per-step noise draws");
+  if (!timesteps || !ac) return fail("ddim_sample: null schedule");
+  std::vector<float> coef((size_t)n * 8, 0.f);
+  if (ddim_coefficients(timesteps, n, ac, n_train, eta, coef.data())) return -1;
+  if (sampler_begin(z_init, cond, B, T, h, w, st)) return -1;
+  UProgram* up = active;
+  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, st)) return -1;
+  // the update reads the noise whenever it has a pointer: only the stochastic variant gets step i's draw (row i)
+  if (loop_replay(*this, up, SAMPLER_DDIM, 0, n, eta > 0.f ? noise : nullptr, 0, st)) return -1;
   B2V_CUDA(cudaMemcpyAsync(z_out, up->x_in, up->numel * 4, cudaMemcpyDeviceToDevice, st));
   if (nan_flag) B2V_CUDA(cudaMemcpyAsync(nan_flag, up->nan_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
   return check_launches("ddim_sample");
@@ -793,17 +813,9 @@ int UNet::dpmpp_sample(const float* z_init, const float* cond, float* z_out, int
     up->x0_prev = (float*)up->ds.alloc(up->numel * 4);
     if (!up->x0_prev) return fail("out of device memory (DPM-Solver++ x0 buffer)");
   }
-  std::vector<long long> ts(timesteps, timesteps + n);
-  B2V_CUDA(cudaMemcpyAsync(up->t_table, ts.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, st));
-  B2V_CUDA(cudaMemcpyAsync(up->coef_table, coef.data(), sizeof(float) * 8 * n, cudaMemcpyHostToDevice, st));
-  if (sde) {  // step i's draw is row i of the caller's buffer (the last row is not read: its c is 0)
-    SamplerCtl c{};
-    c.noise = noise;
-    B2V_CUDA(cudaMemcpyAsync(up->ctl, &c, sizeof c, cudaMemcpyHostToDevice, st));
-  }
-  if (temb_tables(up, n, st)) return -1;
-  for (int i = 0; i < n; ++i)
-    if (up->dpmpp.run(st)) return -1;
+  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, st)) return -1;
+  // step i's draw is row i of the caller's buffer (the last row is not read: its c is 0)
+  if (loop_replay(*this, up, SAMPLER_DPMPP, 0, n, sde ? noise : nullptr, 0, st)) return -1;
   B2V_CUDA(cudaMemcpyAsync(z_out, up->x_in, up->numel * 4, cudaMemcpyDeviceToDevice, st));
   if (nan_flag) B2V_CUDA(cudaMemcpyAsync(nan_flag, up->nan_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
   return check_launches("dpmpp_sample");
@@ -826,26 +838,13 @@ int UNet::ddpm_run(const float* coef, int n, int first, int count, const float* 
       ts[s] = n - 1 - s;
       for (int j = 0; j < 8; ++j) rows[(size_t)s * 8 + j] = coef[(size_t)(n - 1 - s) * 8 + j];
     }
-    B2V_CUDA(cudaMemcpyAsync(up->t_table, ts.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, st));
-    B2V_CUDA(cudaMemcpyAsync(up->coef_table, rows.data(), sizeof(float) * 8 * n, cudaMemcpyHostToDevice, st));
-    if (temb_tables(up, n, st)) return -1;
+    if (loop_tables(*this, up, ts, rows, st)) return -1;
     up->loop_n = n;
   } else if (n != up->loop_n) {
     return fail("ddpm_run: loop length changed between chunks");
   }
   if (count == 0) return 0;
-  {  // this chunk's noise source; step / nan_flag are owned by the device (offsetof: the first two ints stay untouched)
-    SamplerCtl c{};
-    c.noise_first = first;
-    c.noise = noise;
-    c.seed = seed;
-    const size_t off = offsetof(SamplerCtl, noise_first);
-    B2V_CUDA(cudaMemcpyAsync((char*)up->ctl + off, (const char*)&c + off, sizeof(SamplerCtl) - off,
-                             cudaMemcpyHostToDevice, st));
-  }
-  up->temb = TembSource{up->proj_all, 0, up->step_dev, proj_rows};
-  for (int i = 0; i < count; ++i)
-    if (up->ddpm.run(st)) return -1;
+  if (loop_replay(*this, up, SAMPLER_DDPM, first, count, noise, seed, st)) return -1;  // this chunk's noise source
   up->loop_pos = first + count;
   return check_launches("ddpm_run");
 }
@@ -861,8 +860,8 @@ int UNet::ddpm_step(long long t, const float* coef, const float* noise, cudaStre
   UProgram* up = active;
   if (!up) return fail("ddpm_step: call b2v_sampler_begin first");
   if (!noise || !coef) return fail("ddpm_step: null noise / coefficients");
-  launch_set_t(up->t_dev, nullptr, nullptr, t, up->B, st);
-  up->temb = TembSource{up->proj, proj_rows, nullptr, 0};
+  launch_set_t(up->t_dev, t, up->B, st);
+  forward_temb(*up);
   if (up->fwd.run(st)) return -1;
   Coef8 c8;
   for (int i = 0; i < 8; ++i) c8.v[i] = coef[i];

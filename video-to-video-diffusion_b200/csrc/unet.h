@@ -28,14 +28,14 @@ struct ULevel {
   bool has_resample = false;
 };
 
+enum { SAMPLER_DDIM = 0, SAMPLER_DDPM = 1, SAMPLER_DPMPP = 2, SAMPLER_KINDS = 3 };  // as b2v_sampler_cfg.sampler
 struct UProgram {
   int B = 0, T = 0, h = 0, w = 0;
   long long numel = 0;
   DeviceStore ds;
   Pool pool;
   std::vector<Op> core;
-  Program fwd, ddim, ddpm;  // one U-Net evaluation | + DDIM update + advance | + DDPM update + advance
-  Program dpmpp;            // + DPM-Solver++(2M) update + advance
+  Program fwd, loop[SAMPLER_KINDS];  // one U-Net evaluation | per sampler: core without time_embed + update + advance
   float *x_in = nullptr, *c_in = nullptr, *eps = nullptr;
   float* x0_prev = nullptr;  // previous step's data prediction (DPM-Solver++), allocated by the first dpmpp_sample
   long long *t_dev = nullptr, *t_table = nullptr;
@@ -45,11 +45,10 @@ struct UProgram {
   float *coef_table = nullptr, *silu_temb = nullptr, *proj = nullptr;
   stat_t* stats = nullptr;
   size_t stats_cap = 0;
-  TembSource temb;            // set before every run: per-sample table (forward) or all-steps table (DDIM graph)
-  float *silu_all = nullptr, *proj_all = nullptr;  // time embedding of every DDIM step, computed once per sample() call
+  TembSource temb;            // set before every run: per-sample table (forward) or all-steps table (loop programs)
+  float *silu_all = nullptr, *proj_all = nullptr;  // time embedding of every loop step, computed once per loop
   int all_cap = 0;
   long long stamp = 0;  // last use (least-recently-used program is evicted when the cache is full)
-  int desc_rows = 0;  // rows of one time-embedding projection table (= UNet::proj_rows)
 };
 
 enum { ATTN_REFERENCE = 0, ATTN_SOFTMAX = 1 };  // b2v_unet_set_attention modes
@@ -78,6 +77,7 @@ struct UNet {
   UProgram* program(int B, int T, int h, int w);
   int forward(const float* x, const long long* t, const float* c, float* eps_out, int B, int T, int h, int w,
               cudaStream_t st);
+  void forward_temb(UProgram& up) const { up.temb = TembSource{up.proj, proj_rows, nullptr, 0}; }  // before up.fwd
   int sampler_begin(const float* z_init, const float* cond, int B, int T, int h, int w, cudaStream_t st);
   int ddim_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
                   const long long* timesteps, int n, const float* ac, int n_train, float eta, const float* noise,
@@ -92,7 +92,6 @@ struct UNet {
                cudaStream_t st);
   int ddpm_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w, const float* coef,
                   int n, const float* noise, unsigned long long seed, cudaStream_t st);
-  int temb_tables(UProgram* up, int n, cudaStream_t st);  // time embedding of every loop step from up->t_table
   int sampler_end(float* z_out, cudaStream_t st);
   ~UNet();
 };

@@ -30,6 +30,43 @@ def _gaussian_weight(d, h, w):
     return g(d)[:, None, None] * g(h)[None, :, None] * g(w)[None, None, :]
 
 
+def _timesteps(n_train, num_inference_steps):
+    """every (T // n)-th training step, plus T-1 if the stride missed it, descending: n (+1) evaluations"""
+    ts = np.arange(0, n_train, n_train // num_inference_steps)
+    if ts[-1] != n_train - 1:
+        ts = np.append(ts, n_train - 1)
+    return ts[::-1]
+
+
+def _schedule(diffusion, num_inference_steps):
+    """(timesteps, alphas_cumprod) of a DDIM / DPM-Solver++ loop: contiguous int64 array, fp32 CPU tensor"""
+    ts = np.ascontiguousarray(_timesteps(diffusion.timesteps, num_inference_steps), dtype=np.int64)
+    return ts, diffusion.alphas_cumprod.detach().float().cpu().contiguous()
+
+
+def _native_sample(smp, entry, shape, conditioning, device, ts, acp, args, draw_noise):
+    """the whole loop as one call of b2v_<entry> on a native UNet3D; RNG order: z, then one randn_like per step if
+    draw_noise.  args are the entry's own arguments between n_train and noise."""
+    shape, dev = check_sampler_args(smp.model, shape, conditioning, device)  # ValueError before any C call
+    z = torch.randn(shape, device=dev)
+    cond = conditioning.detach().to(dev, torch.float32).contiguous()
+    B, _, T, h, w = shape
+    if z.numel() == 0:
+        return z
+    n = len(ts)
+    noise = torch.stack([torch.randn_like(z) for _ in range(n)]).contiguous() if draw_noise else None
+    out = torch.empty_like(z)
+    flag = torch.zeros(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(getattr(_lib.lib(), "b2v_" + entry)(
+            smp.model.native(dev), _lib.dptr(z), _lib.dptr(cond), _lib.dptr(out), B, T, h, w,
+            ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), n,
+            ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)), acp.numel(), *args,
+            _lib.dptr(noise), _lib.dptr(flag, torch.int32), _lib.stream()), entry)
+    smp.last_nan_flag = flag  # device tensor; .item() it to learn whether a NaN/Inf guard fired
+    return out
+
+
 def _starts(full, size, stride):
     return sorted(set(list(range(0, full - size + 1, stride)) + [max(0, full - size)]))
 
@@ -83,40 +120,17 @@ class DDIMSampler(_Stitching):
         self.diffusion, self.model, self.timesteps = diffusion, model, diffusion.timesteps
 
     def _get_timesteps(self, num_inference_steps):
-        """every (T // n)-th training step, plus T-1 if the stride missed it, descending: n (+1) evaluations"""
-        ts = np.arange(0, self.timesteps, self.timesteps // num_inference_steps)
-        if ts[-1] != self.timesteps - 1:
-            ts = np.append(ts, self.timesteps - 1)
-        return ts[::-1]
+        return _timesteps(self.timesteps, num_inference_steps)
 
     @torch.no_grad()
     def sample(self, shape, conditioning, num_inference_steps, device, eta=0.0, progress=True):
-        ts = np.ascontiguousarray(self._get_timesteps(num_inference_steps), dtype=np.int64)
-        n = len(ts)
-        acp = self.diffusion.alphas_cumprod.detach().float().cpu().contiguous()
+        ts, acp = _schedule(self.diffusion, num_inference_steps)
         if not _is_native(self.model):
             dev = torch.device(device)
             z = torch.randn(shape, device=dev)
             return self._sample_generic(z, conditioning.detach().to(dev, torch.float32).contiguous(), ts, acp, eta)
-        shape, dev = check_sampler_args(self.model, shape, conditioning, device)  # ValueError before any C call
-        z = torch.randn(shape, device=dev)
-        cond = conditioning.detach().to(dev, torch.float32).contiguous()
-        B, _, T, h, w = shape
-        if z.numel() == 0:
-            return z
-        noise = None
-        if eta > 0:  # the reference draws one randn_like per step; nothing else touches the RNG in between
-            noise = torch.stack([torch.randn_like(z) for _ in range(n)]).contiguous()
-        out = torch.empty_like(z)
-        flag = torch.zeros(1, dtype=torch.int32, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(_lib.lib().b2v_ddim_sample(
-                self.model.native(dev), _lib.dptr(z), _lib.dptr(cond), _lib.dptr(out), B, T, h, w,
-                ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), n,
-                ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)), acp.numel(), float(eta),
-                _lib.dptr(noise), _lib.dptr(flag, torch.int32), _lib.stream()), "ddim_sample")
-        self.last_nan_flag = flag  # device tensor; .item() it only if you want the reference's error log
-        return out
+        # the reference draws one randn_like per step when eta > 0; nothing else touches the RNG in between
+        return _native_sample(self, "ddim_sample", shape, conditioning, device, ts, acp, (float(eta),), eta > 0)
 
     def _sample_generic(self, z, cond, ts, acp, eta):
         """any callable model(z, t, c): Python loop, fused update kernel per step"""
@@ -173,38 +187,23 @@ class DPMSolverSampler(_Stitching):
         self.diffusion, self.model, self.timesteps = diffusion, model, diffusion.timesteps
 
     def _get_timesteps(self, num_inference_steps):
-        return DDIMSampler._get_timesteps(self, num_inference_steps)
+        return _timesteps(self.timesteps, num_inference_steps)
 
     @torch.no_grad()
     def sample(self, shape, conditioning, num_inference_steps, device, order=2, stochastic=False, progress=True):
         if order not in (1, 2):
             raise ValueError(f"DPMSolverSampler: order must be 1 or 2, got {order}")
-        ts = np.ascontiguousarray(self._get_timesteps(num_inference_steps), dtype=np.int64)
-        n = len(ts)
-        acp = self.diffusion.alphas_cumprod.detach().float().cpu().contiguous()
-        native = _is_native(self.model)
-        if native:
-            shape, dev = check_sampler_args(self.model, shape, conditioning, device)  # ValueError before any C call
-        else:
-            dev = torch.device(device)
+        ts, acp = _schedule(self.diffusion, num_inference_steps)
+        if _is_native(self.model):
+            return _native_sample(self, "dpmpp_sample", shape, conditioning, device, ts, acp,
+                                  (int(order), int(stochastic)), stochastic)
+        dev = torch.device(device)
         z = torch.randn(shape, device=dev)
         cond = conditioning.detach().to(dev, torch.float32).contiguous()
         if z.numel() == 0:
             return z
-        noise = torch.stack([torch.randn_like(z) for _ in range(n)]).contiguous() if stochastic else None
-        if not native:
-            return self._sample_generic(z, cond, ts, dpmpp_coefficients(ts, acp, order, stochastic).to(dev), noise)
-        B, _, T, h, w = shape
-        out = torch.empty_like(z)
-        flag = torch.zeros(1, dtype=torch.int32, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(_lib.lib().b2v_dpmpp_sample(
-                self.model.native(dev), _lib.dptr(z), _lib.dptr(cond), _lib.dptr(out), B, T, h, w,
-                ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), n,
-                ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)), acp.numel(), int(order), int(stochastic),
-                _lib.dptr(noise), _lib.dptr(flag, torch.int32), _lib.stream()), "dpmpp_sample")
-        self.last_nan_flag = flag  # device tensor; .item() it to learn whether a NaN/Inf guard fired
-        return out
+        noise = torch.stack([torch.randn_like(z) for _ in range(len(ts))]).contiguous() if stochastic else None
+        return self._sample_generic(z, cond, ts, dpmpp_coefficients(ts, acp, order, stochastic).to(dev), noise)
 
     def _sample_generic(self, z, cond, ts, rows, noise):
         """any callable model(z, t, c): Python loop, the update kernel per step (in place on z)"""

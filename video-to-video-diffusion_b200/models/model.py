@@ -102,10 +102,8 @@ class VideoToVideoDiffusion(nn.Module):
         cfg = _lib.SamplerCfg()
         keep = []  # host tables must outlive the call
         if sampler != "ddpm":
-            from ..inference.sampler import DDIMSampler
-            ts = np.ascontiguousarray(DDIMSampler(self.diffusion, self.unet)._get_timesteps(num_inference_steps),
-                                      dtype=np.int64)
-            acp = self.diffusion.alphas_cumprod.detach().float().cpu().contiguous()
+            from ..inference.sampler import _schedule
+            ts, acp = _schedule(self.diffusion, num_inference_steps)
             keep += [ts, acp]
             code = {"ddim": 0, "dpmpp_2m": 2, "dpmpp_2m_sde": 3}[sampler]
             cfg.sampler, cfg.n, cfg.n_train, cfg.eta = code, len(ts), acp.numel(), 0.0
