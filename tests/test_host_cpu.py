@@ -232,6 +232,8 @@ def test_unsupported_configs_fail_at_construction():
         UNet3D(latent_dim=4, model_channels=96)
     with pytest.raises(ValueError, match="latent_dim"):
         UNet3D(latent_dim=12, model_channels=64, channel_mult=(1,), attention_levels=[])
+    with pytest.raises(ValueError, match="2048"):
+        UNet3D(latent_dim=4, model_channels=1088, channel_mult=(1, 2), attention_levels=[])
     with pytest.raises(ValueError, match="multiple of 64"):
         VideoVAE(1, 4, 32, 1.0)
     UNet3D(latent_dim=4, model_channels=192, channel_mult=(1, 2), num_res_blocks=1, attention_levels=[1])  # 24 ch / group

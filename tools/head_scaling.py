@@ -18,5 +18,5 @@ for cout in (1, 8):
             conv(x16, out_fp32=True)
         e1.record(); torch.cuda.synchronize()
         pos = B * D * H * H
-        print(f"dbg={os.environ.get('B2V_TAP_DEBUG','0')} cout={cout} positions={pos/1e6:.2f}M  {e0.elapsed_time(e1)/5:.4f} ms  P={27*cout*pos*4/1e6:.0f} MB in={pos*256/1e6:.0f} MB")
+        print(f"cout={cout} positions={pos/1e6:.2f}M  {e0.elapsed_time(e1)/5:.4f} ms  P={27*cout*pos*4/1e6:.0f} MB in={pos*256/1e6:.0f} MB")
         del x16, conv

@@ -23,4 +23,4 @@ tu = timeit(lambda: m.unet(x, t, c), N)
 td = timeit(lambda: m.vae.decode(x), 5)
 v = torch.rand((B, 1, 8, 192, 192), device=dev) * 2 - 1
 te = timeit(lambda: m.vae.encode(v), 5)
-print(f"PDL={'off' if os.environ.get('B2V_NO_PDL') else 'on'} B={B}: unet_step {tu:.3f} ms  decode {td:.3f} ms  encode {te:.3f} ms")
+print(f"B={B}: unet_step {tu:.3f} ms  decode {td:.3f} ms  encode {te:.3f} ms")

@@ -297,8 +297,7 @@ static void out_grid(const ConvLayer& L, int D, int H, int W, int& gD, int& gH, 
 }
 
 int conv_splitk_factor(const ConvLayer& L, int N, int D, int H, int W) {
-  static const bool off = getenv("B2V_NO_SPLITK") != nullptr;
-  if (off || L.bn < 64 || L.kind == CONV_UPT || L.cout % 8) return 1;
+  if (L.bn < 64 || L.kind == CONV_UPT || L.cout % 8) return 1;
   int gD, gH, gW, bw, bh, bd;
   out_grid(L, D, H, W, gD, gH, gW);
   choose_box(gW, gH, gD, bw, bh, bd);
@@ -329,8 +328,7 @@ static inline long long tap_slice_tiles(int H, int W) { return ((long long)H * W
 static inline long long tap_pairs(int N, int D, int H, int W) { return (tap_slice_tiles(H, W) * D * N + 1) / 2; }
 
 size_t conv_tap_ws_bytes(const ConvLayer& L, int N, int D, int H, int W) {
-  static const bool off = getenv("B2V_NO_TAPGEMM") != nullptr;
-  if (!L.tapgemm || off) return 0;
+  if (!L.tapgemm) return 0;
   return (size_t)9 * L.cout * (size_t)(tap_pairs(N, D, H, W) * 256) * sizeof(float);
 }
 
@@ -492,9 +490,8 @@ int conv_plan(ConvPlan& P, const ConvLayer& L, const __half* in0, const __half* 
   }
   long long total = (long long)p.tiles_w * p.tiles_h * p.tiles_d * N * p.nclass * p.n_tiles;
   const int sms = device_sm_count();
-  static const bool no_swap = getenv("B2V_NO_SWAP") != nullptr;
   const int tiles_per_sample = p.tiles_w * p.tiles_h * p.tiles_d;
-  P.swapped = !no_swap && L.cout == 128 && L.bn == 128 && out_mode == OUT_CL16 && act == ACT_NONE &&
+  P.swapped = L.cout == 128 && L.bn == 128 && out_mode == OUT_CL16 && act == ACT_NONE &&
               (tiles_per_sample % 2 == 0) && (!stats || p.cpg <= 32);
   if (P.swapped) total /= 2;
   if (splitk_ws && !P.swapped && out_mode == OUT_CL16 && act == ACT_NONE) {
@@ -534,9 +531,8 @@ int conv_plan(ConvPlan& P, const ConvLayer& L, const __half* in0, const __half* 
 
 void conv_launch(const ConvPlan& P, cudaStream_t st) {
   if (P.tapgemm) {
-    static const int dbg = getenv("B2V_TAP_DEBUG") ? atoi(getenv("B2V_TAP_DEBUG")) : 0;  // 1: GEMM only, 2: stencil only
-    if (dbg != 2) launch_k(conv_igemm_t_kernel<1>, dim3(P.grid), dim3(ConvCfgT::threads(1)), ConvCfgT::SMEM, st, P.p);
-    if (dbg != 1) launch_head_stencil(P.st.P, P.st.bias, P.st.out, P.st.N, P.st.cout, P.st.D, P.st.H, P.st.W, P.st.row_stride,
+    launch_k(conv_igemm_t_kernel<1>, dim3(P.grid), dim3(ConvCfgT::threads(1)), ConvCfgT::SMEM, st, P.p);
+    launch_head_stencil(P.st.P, P.st.bias, P.st.out, P.st.N, P.st.cout, P.st.D, P.st.H, P.st.W, P.st.row_stride,
                         P.st.slice_stride, P.st.act, st);
     return;
   }

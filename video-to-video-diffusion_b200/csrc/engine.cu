@@ -241,7 +241,7 @@ stat_t* Builder::new_stats(int G) {
 }
 
 Act Builder::conv(const std::string& name, const ConvLayer& L, const Act& in0, const Act* in1, stat_t* stats,
-                  int groups, float* out_fp32, int act, const float* bias_override) {
+                  int groups, float* out_fp32, int act) {
   Act out;
   int oD = in0.D, oH = in0.H, oW = in0.W;
   if (L.kind == CONV_DOWN) {
@@ -288,10 +288,6 @@ Act Builder::conv(const std::string& name, const ConvLayer& L, const Act& in0, c
     fail(name + ": " + err);
     ok = false;
     return out;
-  }
-  if (bias_override) {
-    P.p.bias = bias_override;
-    P.fin.bias = bias_override;
   }
   Op op;
   op.name = name;

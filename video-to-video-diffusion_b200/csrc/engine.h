@@ -122,7 +122,7 @@ struct Builder {
   stat_t* new_stats(int G);
   // out_fp32 != nullptr: NCDHW fp32 head; otherwise returns a fresh cl16 activation
   Act conv(const std::string& name, const ConvLayer& L, const Act& in0, const Act* in1, stat_t* stats, int groups,
-           float* out_fp32 = nullptr, int act = ACT_NONE, const float* bias_override = nullptr);
+           float* out_fp32 = nullptr, int act = ACT_NONE);
   // temb_off >= 0: add row offset temb_off of the time-embedding table (*temb_src) after the SiLU (mode 0)
   void gn_apply(const std::string& name, Act& y, const stat_t* stats_in, const GNW& g, int temb_off, const Act* res,
                 int mode, stat_t* stats_out, int G_out);

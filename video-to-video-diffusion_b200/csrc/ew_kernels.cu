@@ -204,38 +204,30 @@ void launch_gn_apply(const __half* y, __half* out, const stat_t* stats_in, const
   const int C8 = C / 8;
   const int R = C8 >= 256 ? 1 : 256 / C8;
   const int threads = C8 * R;
-  static const int U = getenv("B2V_GN_UNROLL") ? atoi(getenv("B2V_GN_UNROLL")) : 4;
+  constexpr int U = 4;
   long long want = (S + U * R - 1) / (U * R);
   // 3 CTAs per SM over the whole launch = one resident wave (72-80 registers x 256 threads): few long-lived CTAs
   // amortise the per-CTA prologue (statistics -> scale / shift) and leave no ragged last wave.  Measured against 8 per
-  // SM: -12 % on the U-Net's GroupNorm-apply total, -3 % on the decoder's (B2V_GN_CTAS_PER_SM overrides for A/B runs).
-  static const int per_sm_env = getenv("B2V_GN_CTAS_PER_SM") ? atoi(getenv("B2V_GN_CTAS_PER_SM")) : 0;
+  // SM: -12 % on the U-Net's GroupNorm-apply total, -3 % on the decoder's.
   // the statistics-producing variants hold 16 more accumulators and fit 2 CTAs per SM
-  const int per_sm = per_sm_env ? per_sm_env : ((stats_out || U > 4) ? 2 : 3);
+  const int per_sm = stats_out ? 2 : 3;
   long long cap = (148LL * per_sm + B - 1) / B;
   int blocks = (int)(want < cap ? want : cap);
   if (blocks < 1) blocks = 1;
   const size_t smem = stats_out ? (size_t)(R + 1) * 2 * C * sizeof(float) : 0;
-#define GN_LAUNCH(UU, MM, SS)                                                                                     \
-  launch_k(gn_apply_kernel<UU, MM, SS>, dim3(dim3(blocks, B)), dim3(threads), smem, st, y, out, stats_in, gamma, beta, temb, temb_stride, \
+#define GN_LAUNCH(MM, SS)                                                                                         \
+  launch_k(gn_apply_kernel<U, MM, SS>, dim3(dim3(blocks, B)), dim3(threads), smem, st, y, out, stats_in, gamma, beta, temb, temb_stride, \
            temb_step, temb_step_stride, res, S, C, G, eps, stats_out, G_out)
-#define GN_DISPATCH(UU)                       \
-  do {                                        \
-    if (mode == 0) {                          \
-      if (stats_out) GN_LAUNCH(UU, 0, true);  \
-      else GN_LAUNCH(UU, 0, false);           \
-    } else if (mode == 2) {                   \
-      if (stats_out) GN_LAUNCH(UU, 2, true);  \
-      else GN_LAUNCH(UU, 2, false);           \
-    } else {                                  \
-      if (stats_out) GN_LAUNCH(UU, 1, true);  \
-      else GN_LAUNCH(UU, 1, false);           \
-    }                                         \
-  } while (0)
-  if (U == 8) GN_DISPATCH(8);
-  else if (U == 2) GN_DISPATCH(2);
-  else GN_DISPATCH(4);
-#undef GN_DISPATCH
+  if (mode == 0) {
+    if (stats_out) GN_LAUNCH(0, true);
+    else GN_LAUNCH(0, false);
+  } else if (mode == 2) {
+    if (stats_out) GN_LAUNCH(2, true);
+    else GN_LAUNCH(2, false);
+  } else {
+    if (stats_out) GN_LAUNCH(1, true);
+    else GN_LAUNCH(1, false);
+  }
 #undef GN_LAUNCH
 }
 
@@ -325,59 +317,11 @@ void launch_gn_stats(const __half* x, int B, long long S, int C, int G, stat_t* 
 // TemporalAttention (reference models/unet3d.py:163-194).  The reference's second einsum
 // 'bhqk,bhvc->bhqc' sums k and v independently, so out[b,:,t,h,w] = (sum_k softmax) * sum_t V = sum_t V
 // for every t.  With V = Wv*GN(x)+bv this is  x + Wp*(Wv * sum_t GN(x) + T*bv) + bp.
-// attn_tsum: s[b,p,c] = sum_t GN32(x)[b,t,p,c] = gamma*rstd*(sum_t x - T*mean) + T*beta    (fp16 out)
-// (the C x C product Wp*Wv and the folded bias are built once at weight-load time; the tiny GEMM runs on
-//  the conv kernel); add_bcast_t: x[b,t,p,:] += y[b,p,:].
+// sum_t GN(x) = gamma*rstd*(sum_t x - T*mean) + T*beta per channel.  Wpv = Wp*Wv is built once at weight-load time and
+// the bias T*(Wp*bv) + bp when a program is built for its depth T.  The fold runs fused with the ResBlock tail that
+// precedes every attention block (below: gn_res_tsum, then attn_gemm + add_bcast_t), so the block output is read once.
 // ------------------------------------------------------------------------------------------------
-// one block per (sample, spatial position); thread = (8-channel vector, depth split): the T slices are shared
-// among blockDim/C8 thread groups (was one thread per column walking all T slices: latency-bound at 1.5 TB/s)
-__global__ void attn_tsum_kernel(const __half* __restrict__ x_, const stat_t* __restrict__ stats,
-                                 const float* __restrict__ gamma, const float* __restrict__ beta, __half* s_, int T,
-                                 int P, int C, int G, float eps) {
-  pdl_trigger();
-  pdl_wait();
-  extern __shared__ float sm[];  // [TS][C]
-  const int C8 = C >> 3;
-  const int TS = blockDim.x / C8;
-  const int cv = threadIdx.x % C8, ts = threadIdx.x / C8;
-  const int p = blockIdx.x % P, b = blockIdx.x / P;
-  const uint4* x = reinterpret_cast<const uint4*>(x_) + ((size_t)b * T * P + p) * C8 + cv;
-  const size_t tstride = (size_t)P * C8;
-  float acc[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) acc[j] = 0.f;
-#pragma unroll 4
-  for (int t = ts; t < T; t += TS) {
-    float f[8];
-    h8_to_f(x[t * tstride], f);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] += f[j];
-  }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) sm[ts * C + cv * 8 + j] = acc[j];
-  __syncthreads();
-  if (ts != 0) return;
-  for (int k = 1; k < TS; ++k)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] += sm[k * C + cv * 8 + j];
-  const int cpg = C / G;
-  float sc[8], sh[8], o[8];
-  gn_scale_shift(stats, gamma, beta, b, G, cpg, 1.0 / ((double)T * (double)P * (double)cpg), eps, cv * 8, sc, sh);
-#pragma unroll
-  for (int j = 0; j < 8; ++j) o[j] = fmaf(sc[j], acc[j], (float)T * sh[j]);  // sum_t (sc*x + sh)
-  reinterpret_cast<uint4*>(s_)[((size_t)b * P + p) * C8 + cv] = f_to_h8(o);
-}
-
-void launch_attn_tsum(const __half* x, const stat_t* stats, const float* gamma, const float* beta, __half* s, int B,
-                      int T, int P, int C, int G, float eps, cudaStream_t st) {
-  const int C8 = C / 8;
-  int TS = 256 / C8;
-  if (TS < 1) TS = 1;
-  if (TS > T) TS = T;
-  launch_k(attn_tsum_kernel, dim3(B * P), dim3(C8 * TS), (size_t)TS * C * sizeof(float), st, x, stats, gamma, beta, s,
-           T, P, C, G, eps);
-}
-
+// add_bcast_t: x[b,t,p,:] += y[b,p,:]
 __global__ void add_bcast_t_kernel(__half* x_, const __half* __restrict__ y_, int T, int PC8) {
   pdl_trigger();
   pdl_wait();
@@ -396,7 +340,7 @@ __global__ void add_bcast_t_kernel(__half* x_, const __half* __restrict__ y_, in
   }
 }
 
-void launch_add_bcast_t(__half* x, const __half* y, int B, int T, int P, int C, cudaStream_t st) {
+static void launch_add_bcast_t(__half* x, const __half* y, int B, int T, int P, int C, cudaStream_t st) {
   const int PC8 = P * (C / 8);
   const long long total = (long long)T * PC8;
   int blocks = cdiv(total, 256);
@@ -406,7 +350,7 @@ void launch_add_bcast_t(__half* x, const __half* y, int B, int T, int P, int C, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Fused form of the attention-followed ResBlock tail + TemporalAttention (the block output is read once less):
+// The attention-followed ResBlock tail + TemporalAttention:
 //   gn_res_tsum   : y = silu(GN(y) + res) in place (ResBlock3D tail, mode 1 of gn_apply), statistics of the result for
 //                   the attention's GroupNorm, and the raw depth sums  tsum[b][ts][p][c] = sum_{t in split ts} y[b,t,p,c]
 //                   -- a thread owns one (position, 8-channel vector) and walks the depth axis, so the depth sum is a

@@ -11,8 +11,6 @@ void launch_gn_apply(const __half* y, __half* out, const stat_t* stats_in, const
 void launch_splitk_finalize(const float* ws, long long slab, int nsplit, const float* bias, __half* out, stat_t* stats,
                             int B, long long S, int C, int G, cudaStream_t st);
 void launch_gn_stats(const __half* x, int B, long long S, int C, int G, stat_t* stats, cudaStream_t st);
-void launch_attn_tsum(const __half* x, const stat_t* stats, const float* gamma, const float* beta, __half* s, int B,
-                      int T, int P, int C, int G, float eps, cudaStream_t st);
 // fused attention-followed ResBlock tail + TemporalAttention (see ew_kernels.cu)
 bool attn_fused_supported(int C);
 int attn_tsum_splits(int B, int T, int P, int C);
@@ -22,7 +20,6 @@ void launch_gn_res_tsum(__half* y, const __half* res, const stat_t* stats_in, co
 void launch_attn_proj_add(__half* x, const float* tsum, int TS, const stat_t* stats, const float* gamma,
                           const float* beta, const __half* Wt, const float* bias, __half* g_ws, int B, int T, int P,
                           int C, int G, float eps, cudaStream_t st);
-void launch_add_bcast_t(__half* x, const __half* y, int B, int T, int P, int C, cudaStream_t st);
 void launch_temb(const long long* t_ptr, const float* freqs, const float* W1, const float* b1, const float* W2,
                  const float* b2, float* silu_temb, const float* Wp, const float* bp, float* proj, int rows, int dim,
                  int td, int B, cudaStream_t st);

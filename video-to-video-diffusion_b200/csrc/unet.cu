@@ -30,7 +30,7 @@ static int load_res(ResW& r, const WeightMap& wm, const std::string& pre, int ci
   return 0;
 }
 
-// reference mode: the TemporalAttention fold (see ew_kernels.cu: attn_tsum): Wpv = Wp*Wv, u = Wp*bv (bias = T*u + bp
+// reference mode: the TemporalAttention fold (see ew_kernels.cu): Wpv = Wp*Wv, u = Wp*bv (bias = T*u + bp
 // at plan time).  softmax mode: the qkv conv as it is and the output projection as a dual-source conv over (o, x)
 // with weight [Wp | I_C], whose identity half adds the block input into the fp32 accumulator (the residual).
 static int load_attn(AttnW& a, const WeightMap& wm, const std::string& pre, int C, DeviceStore& ds, int mode) {
@@ -75,8 +75,6 @@ static int load_attn(AttnW& a, const WeightMap& wm, const std::string& pre, int 
     for (int k = 0; k < C; ++k) s += (double)Wp[(size_t)o * C + k] * bv[k];
     a.u[o] = (float)s;
   }
-  std::string err;
-  if (conv_layer_init(a.pv, CONV_K1, Wpv.data(), nullptr, C, 0, C, err)) return fail(pre + ": " + err);
   // transposed fp16 copy for the fused attn_proj_add kernel: Wt[c][co] = Wpv[co][c]
   std::vector<__half> wt((size_t)C * C);
   for (int o = 0; o < C; ++o)
@@ -114,6 +112,10 @@ int UNet::finalize() {
   const b2v_unet_desc& d = desc;
   const int mc = d.model_channels, td = d.time_embed_dim, L = d.latent_dim, NL = d.num_levels;
   if (mc % 64) return fail("model_channels must be a multiple of 64");
+  for (int l = 0; l < NL; ++l)
+    if (mc * d.channel_mult[l] > 2048)
+      return fail("model_channels * channel_mult must be <= 2048 at every level (GroupNorm kernels: <= 256 threads of "
+                  "8 channels per row)");
   if (2 * L * 3 > 64) return fail("latent_dim too large for the packed conv_in (2*latent_dim*3 must be <= 64)");
   if (td > 4096 || mc > 4096) return fail("time_embed_dim / model_channels too large");
   std::string err;
@@ -195,7 +197,6 @@ int UNet::finalize() {
 UNet::~UNet() {
   progs.clear();
   auto fa = [](AttnW& a) {
-    conv_layer_free(a.pv);
     conv_layer_free(a.qkv);
     conv_layer_free(a.proj);
   };
@@ -222,11 +223,6 @@ UNet::~UNet() {
 }
 
 // ------------------------------------------------------------------ program
-static bool attn_fused(int C) {
-  static const bool off = getenv("B2V_ATTN_UNFUSED") != nullptr;  // A/B switch: the four-launch form
-  return !off && attn_fused_supported(C);
-}
-
 struct UBuild {
   UNet& u;
   UProgram& up;
@@ -237,9 +233,9 @@ struct UBuild {
   }
 
   // ResBlock3D.forward (models/unet3d.py:116-133)
-  // tsum_out != nullptr: the block feeds a TemporalAttention -- its tail also emits the depth sums (fused path)
+  // tsum_out != nullptr: the block feeds a reference-mode TemporalAttention -- its tail also emits the depth sums
   Act res(const std::string& name, const ResW& r, const Act& x, const Act* skip, stat_t** out_stats, int G_out,
-          float** tsum_out = nullptr, int* ts_out = nullptr) {
+          float** tsum_out = nullptr) {
     stat_t* s1 = b.new_stats(r.n1.G);
     Act y1 = b.conv(name + ".conv1", r.conv1, x, skip, s1, r.n1.G);
     Act rr;
@@ -260,7 +256,6 @@ struct UBuild {
         return y2;
       }
       *tsum_out = tsum;
-      *ts_out = TS;
       __half* yp = y2.p;
       const __half* rp = r.has_res ? rr.p : x.p;
       const float *ga = r.n2.gamma, *be = r.n2.beta;
@@ -280,72 +275,41 @@ struct UBuild {
     return y2;
   }
 
-  // TemporalAttention.forward (models/unet3d.py:163-194), folded: x += Wpv * sum_t GN(x) + (T*u + bp)
-  void attn(const std::string& name, const AttnW& a, Act& x, const stat_t* stats_x, float* tsum = nullptr, int TS = 0) {
-    const int B = up.B, T = x.D, P = x.H * x.W, C = x.C;
+  // TemporalAttention.forward (models/unet3d.py:163-194), folded: x += Wpv * sum_t GN(x) + (T*u + bp).  Reference mode
+  // reads the depth sums `tsum` that res() emitted for this block; softmax mode runs the attention as it is.
+  void attn(const std::string& name, const AttnW& a, Act& x, const stat_t* stats_x, float* tsum) {
     if (u.attention == ATTN_SOFTMAX) {
       attn_softmax(name, a, x, stats_x);
       return;
     }
-    if (tsum) {
-      std::vector<float> bias(C, 0.f);
-      for (int i = 0; i < C; ++i) bias[i] = (float)T * a.u[i] + a.bp[i];
-      const float* bias_d = up.ds.upload(bias);
-      if (!bias_d) {
-        b.ok = false;
-        return;
-      }
-      __half* xp = x.p;
-      const __half* wt = a.Wt;
-      const float *ga = a.norm.gamma, *be = a.norm.beta;
-      const int G = a.norm.G;
-      Op op;
-      op.name = name + ".proj_add";
-      op.bytes = (double)B * T * P * C * 2.0 * 2.0;
-      // algorithmic FLOPs of the reference block: qkv (C->3C) and proj (C->C) 1x1 convs over all T positions
-      op.flops = 2.0 * B * T * P * (double)C * (4.0 * C);
-      op.out = xp;
-      op.out_bytes = (size_t)B * T * P * C * 2;
-      op.launches = 2;
-      __half* g_ws = (__half*)(tsum + (size_t)B * TS * P * C);
-      op.run = [=](cudaStream_t st) {
-        launch_attn_proj_add(xp, tsum, TS, stats_x, ga, be, wt, bias_d, g_ws, B, T, P, C, G, 1e-5f, st);
-      };
-      b.ops.push_back(std::move(op));
-      b.pool.put(tsum);
-      return;
-    }
-    Act s = b.alloc(C, 1, x.H, x.W);
-    if (!b.ok) return;
-    {
-      const __half* xp = x.p;
-      __half* sp = s.p;
-      const float *ga = a.norm.gamma, *be = a.norm.beta;
-      const int G = a.norm.G;
-      Op op;
-      op.name = name + ".gn_tsum";
-      op.bytes = (double)B * T * P * C * 2.0;
-      op.run = [=](cudaStream_t st) { launch_attn_tsum(xp, stats_x, ga, be, sp, B, T, P, C, G, 1e-5f, st); };
-      b.ops.push_back(std::move(op));
-    }
-    std::vector<float> bias(a.pv.cout_pad, 0.f);
+    if (!b.ok) return;  // res() could not allocate the depth sums
+    const int B = up.B, T = x.D, P = x.H * x.W, C = x.C;
+    const int TS = attn_tsum_splits(B, T, P, C);
+    std::vector<float> bias(C, 0.f);
     for (int i = 0; i < C; ++i) bias[i] = (float)T * a.u[i] + a.bp[i];
     const float* bias_d = up.ds.upload(bias);
-    Act y = b.conv(name + ".pv_gemm", a.pv, s, nullptr, nullptr, 0, nullptr, ACT_NONE, bias_d);
-    // algorithmic FLOPs of the reference block: qkv (C->3C) and proj (C->C) 1x1 convs over all T positions
-    b.ops.back().flops = 2.0 * B * T * P * (double)C * (4.0 * C);
-    b.free(s);
-    if (!b.ok) return;
-    {
-      __half* xp = x.p;
-      const __half* yp = y.p;
-      Op op;
-      op.name = name + ".add_bcast";
-      op.bytes = (double)B * T * P * C * 2.0 * 2.0;
-      op.run = [=](cudaStream_t st) { launch_add_bcast_t(xp, yp, B, T, P, C, st); };
-      b.ops.push_back(std::move(op));
+    if (!bias_d) {
+      b.ok = false;
+      return;
     }
-    b.free(y);
+    __half* xp = x.p;
+    const __half* wt = a.Wt;
+    const float *ga = a.norm.gamma, *be = a.norm.beta;
+    const int G = a.norm.G;
+    Op op;
+    op.name = name + ".proj_add";
+    op.bytes = (double)B * T * P * C * 2.0 * 2.0;
+    // algorithmic FLOPs of the reference block: qkv (C->3C) and proj (C->C) 1x1 convs over all T positions
+    op.flops = 2.0 * B * T * P * (double)C * (4.0 * C);
+    op.out = xp;
+    op.out_bytes = (size_t)B * T * P * C * 2;
+    op.launches = 2;
+    __half* g_ws = (__half*)(tsum + (size_t)B * TS * P * C);
+    op.run = [=](cudaStream_t st) {
+      launch_attn_proj_add(xp, tsum, TS, stats_x, ga, be, wt, bias_d, g_ws, B, T, P, C, G, 1e-5f, st);
+    };
+    b.ops.push_back(std::move(op));
+    b.pool.put(tsum);
   }
 
   // softmax attention over the T depth tokens: h = GN(x); q, k, v = qkv(h); o = softmax(q k^T / sqrt(hd)) v per
@@ -468,6 +432,7 @@ static int build_unet_program(UNet& u, UProgram& up) {
 
   UBuild ub(u, up);
   Builder& b = ub.b;
+  const bool ref_attn = u.attention == ATTN_REFERENCE;  // attention-followed ResBlocks emit the depth sums
   {
     float* stats = reinterpret_cast<float*>(up.stats);
     const size_t bytes = up.stats_cap * sizeof(stat_t);
@@ -514,13 +479,11 @@ static int build_unet_program(UNet& u, UProgram& up) {
       const std::string nm = "down" + std::to_string(l) + "." + std::to_string(i);
       const bool at = !lv.attn.empty();
       float* tsum = nullptr;
-      int TS = 0;
-      const bool fz = at && u.attention == ATTN_REFERENCE && attn_fused(lv.attn[i].C);
       Act nxt = ub.res(nm, lv.res[i], cur, nullptr, at ? &cur_stats : nullptr, at ? lv.attn[i].norm.G : 0,
-                       fz ? &tsum : nullptr, &TS);
+                       at && ref_attn ? &tsum : nullptr);
       b.free(cur);
       cur = nxt;
-      if (at) ub.attn(nm + ".attn", lv.attn[i], cur, cur_stats, tsum, TS);
+      if (at) ub.attn(nm + ".attn", lv.attn[i], cur, cur_stats, tsum);
     }
     skips.push_back(cur);
     cur_is_skip = true;
@@ -532,12 +495,10 @@ static int build_unet_program(UNet& u, UProgram& up) {
   if (!b.ok) return -1;
   {
     float* tsum = nullptr;
-    int TS = 0;
-    Act nxt = ub.res("mid1", u.mid1, cur, nullptr, &cur_stats, u.mid_attn.norm.G,
-                     (u.attention == ATTN_REFERENCE && attn_fused(u.mid_attn.C)) ? &tsum : nullptr, &TS);
+    Act nxt = ub.res("mid1", u.mid1, cur, nullptr, &cur_stats, u.mid_attn.norm.G, ref_attn ? &tsum : nullptr);
     if (!cur_is_skip) b.free(cur);
     cur = nxt;
-    ub.attn("mid.attn", u.mid_attn, cur, cur_stats, tsum, TS);
+    ub.attn("mid.attn", u.mid_attn, cur, cur_stats, tsum);
     nxt = ub.res("mid2", u.mid2, cur, nullptr, nullptr, 0);
     b.free(cur);
     cur = nxt;
@@ -552,20 +513,19 @@ static int build_unet_program(UNet& u, UProgram& up) {
       const int Go = at ? lv.attn[i].norm.G : (last ? u.out_norm.G : 0);
       Act nxt;
       float* tsum = nullptr;
-      int TS = 0;
-      float** tso = (at && u.attention == ATTN_REFERENCE && attn_fused(lv.attn[i].C)) ? &tsum : nullptr;
+      float** tso = at && ref_attn ? &tsum : nullptr;
       if (i == 0) {
         Act skip = skips.back();
         skips.pop_back();
-        nxt = ub.res(nm, lv.res[i], cur, &skip, so, Go, tso, &TS);
+        nxt = ub.res(nm, lv.res[i], cur, &skip, so, Go, tso);
         b.free(skip);
       } else {
-        nxt = ub.res(nm, lv.res[i], cur, nullptr, so, Go, tso, &TS);
+        nxt = ub.res(nm, lv.res[i], cur, nullptr, so, Go, tso);
       }
       b.free(cur);
       cur = nxt;
       if (at) {
-        ub.attn(nm + ".attn", lv.attn[i], cur, cur_stats, tsum, TS);
+        ub.attn(nm + ".attn", lv.attn[i], cur, cur_stats, tsum);
         if (last) {  // conv_out's GroupNorm needs statistics of the post-attention tensor
           cur_stats = b.new_stats(u.out_norm.G);
           const __half* xp = cur.p;

@@ -14,7 +14,6 @@ struct ResW {  // ResBlock3D (models/unet3d.py:77-133)
 };
 struct AttnW {  // TemporalAttention (models/unet3d.py:136-194): folded (reference mode) or qkv / proj (softmax mode)
   GNW norm;
-  ConvLayer pv;
   ConvLayer qkv;   // softmax mode: the qkv 1x1 conv, C -> 3C
   ConvLayer proj;  // softmax mode: dual-source 1x1 conv over (o, x) with weight [Wproj | I_C], bias bproj
   __half* Wt = nullptr;  // [c][co] fp16 transpose of the folded Wp*Wv (fused attn_proj_add path; owned by UNet::ds)

@@ -113,6 +113,9 @@ class UNet3D(nn.Module):
             raise ValueError(f"UNet3D: latent_dim = {latent_dim} too large for the packed conv_in (<= 10)")
         if not 1 <= nl <= 8 or num_res_blocks < 1:
             raise ValueError("UNet3D: 1..8 levels and at least one ResBlock per level")
+        if model_channels * max(channel_mult) > 2048:
+            raise ValueError(f"UNet3D: model_channels * max(channel_mult) = {model_channels * max(channel_mult)} is "
+                             "above 2048 (the GroupNorm kernels run one 8-channel vector per thread, <= 256 threads)")
 
         def stage(cin, cout, attn):
             layers = [ResBlock3D(cin, cout, time_embed_dim)]
