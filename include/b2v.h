@@ -169,6 +169,24 @@ typedef struct {
 } b2v_sampler_cfg;
 int b2v_generate(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const float* v_in, const float* z_init,
                  float* v_out, int B, int T_in, int T_out, int H, int W, int* nan_flag, void* stream);
+/* Ensemble generation (not in the reference): K >= 2 samples of each of the B inputs and their per-voxel statistics,
+ * in one call with no host synchronisation.  Member m = k*B + b is sample k of input b (k-major):
+ *   NaN check of v_in -> encode the B inputs once -> guard -> depth upsample once -> guard -> conditioning repeated
+ *   K times -> the sampler at batch K*B -> guard -> decode in K chunks of B (the batch-B decode of b2v_generate) ->
+ *   guard -> b2v_ensemble_stats.
+ *   cfg         : as for b2v_generate at batch K*B (SDE noise [n][K*B*numel], DDPM with noise == NULL: device Philox)
+ *   z_init      : (K*B, L, T_out, H/4, W/4)
+ *   members_out : (K, B, Cin, T_out, H, W), or NULL: the members are decoded into the U-Net object's scratch
+ *   mean_out, std_out : (B, Cin, T_out, H, W)
+ *   *nan_flag (DEVICE int, may be NULL) = the OR of all NaN/Inf checkpoints, as in b2v_generate.
+ * Every argument is checked before the first device call.
+ * b2v_ensemble_stats: members DEVICE fp32 [K][n] -> mean, std DEVICE fp32 [n]: mean = sum/K and the unbiased
+ *   std = sqrt(max(0, (sum x^2 - sum x * mean) / (K - 1))), both sums in fp64 over k = 0..K-1 in order (bitwise
+ *   reproducible); K >= 2.                                                                                       */
+int b2v_generate_ensemble(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const float* v_in, const float* z_init,
+                          int K, float* members_out, float* mean_out, float* std_out, int B, int T_in, int T_out, int H,
+                          int W, int* nan_flag, void* stream);
+int b2v_ensemble_stats(const float* members, float* mean, float* stdev, int K, long long n, void* stream);
 
 /* models/diffusion.py:81-190  training forward (no backward): q_sample and the per-sample terms of training_loss.
  *   b2v_q_sample : z_t = sqrt_alphas_cumprod[t_b] * z_0 + sqrt_one_minus_alphas_cumprod[t_b] * noise
@@ -188,7 +206,8 @@ int b2v_upsample_depth(const float* in, float* out, int BC, int Din, int Dout, i
 
 /* inference/sampler.py:379-451  sliding-window stitching: acc[bc, d0+d, h0+h, w0+w] += patch * gd[d]*gh[h]*gw[w],
  * wsum likewise (patch: (BC,pd,ph,pw); acc, wsum: (BC,D,H,W); gd/gh/gw: the separable Gaussian window, device fp32),
- * then acc /= (wsum + 1e-8).  Windows accumulated by concurrent launches must not overlap.                     */
+ * then acc /= (wsum + 1e-8).  Windows accumulated by concurrent launches must not overlap.  wsum may be NULL in
+ * b2v_stitch_accumulate: only acc is written (a second quantity blended with the weights summed by another call). */
 int b2v_stitch_accumulate(const float* patch, float* acc, float* wsum, const float* gd, const float* gh,
                           const float* gw, int BC, int pd, int ph, int pw, int D, int H, int W, int d0, int h0, int w0,
                           void* stream);

@@ -64,6 +64,9 @@ SIGNATURES = {
     "b2v_ddim_timesteps": (c_int, [c_int, c_int, POINTER(c_int64), c_int]),
     "b2v_philox_normal": (c_int, [_P, c_uint64, c_int, c_longlong, _P]),
     "b2v_generate": (c_int, [_P, _P, POINTER(SamplerCfg), _P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "b2v_generate_ensemble": (c_int, [_P, _P, POINTER(SamplerCfg), _P, _P, c_int, _P, _P, _P, c_int, c_int, c_int, c_int,
+                                      c_int, _P, _P]),
+    "b2v_ensemble_stats": (c_int, [_P, _P, _P, c_int, c_longlong, _P]),
     "b2v_q_sample": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_longlong, _P]),
     "b2v_eps_mse_ws_bytes": (c_size_t, [c_int]),
     "b2v_eps_mse": (c_int, [_P, _P, _P, _P, _P, c_size_t, c_int, c_longlong, c_longlong, _P]),

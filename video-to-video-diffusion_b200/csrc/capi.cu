@@ -49,6 +49,102 @@ static int store_weight(WeightMap& wm, bool finalized, const char* key, const fl
   return 0;
 }
 
+// The argument checks of b2v_generate / b2v_generate_ensemble, all made before the first device call.
+static int check_generate_args(const std::string& who, const b2v_sampler_cfg* cfg, int B, int T_in, int T_out, int H,
+                               int W) {
+  if (B < 0 || T_in < 1 || T_out < 1 || H < 4 || W < 4 || H % 4 || W % 4) return fail(who + ": bad shape");
+  if (cfg->sampler < 0 || cfg->sampler > 3)
+    return fail(who + ": unknown sampler (0 = ddim, 1 = ddpm, 2 = dpmpp_2m, 3 = dpmpp_2m_sde)");
+  if (cfg->sampler >= 2) {  // reject a bad DPM-Solver++ configuration before the encoder is launched
+    if (cfg->sampler == 3 && !cfg->noise) return fail(who + ": dpmpp_2m_sde needs the per-step noise draws");
+    if (cfg->n < 1 || cfg->n > 4096) return fail(who + ": 1 <= n <= 4096 timesteps");
+    std::vector<float> rows((size_t)cfg->n * 8);
+    if (dpmpp_coefficients((const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod, cfg->n_train, 2,
+                           cfg->sampler == 3, rows.data()))
+      return -1;
+  }
+  return 0;
+}
+
+// b2v_unet::gen_ws holds at least `need` bytes (grown on demand; the old buffer may be in use by queued work)
+static int gen_workspace(b2v_unet* u, size_t need, cudaStream_t st) {
+  if (need <= u->gen_cap) return 0;
+  B2V_CUDA(cudaStreamSynchronize(st));
+  if (u->gen_ws) cudaFree(u->gen_ws);
+  u->gen_ws = nullptr;
+  u->gen_cap = 0;
+  B2V_CUDA(cudaMalloc(&u->gen_ws, need));
+  u->gen_cap = need;
+  return 0;
+}
+
+// The front of generate(), shared by b2v_generate (K = 1) and b2v_generate_ensemble: NaN check of v_in -> encode the B
+// inputs -> guard -> depth upsample -> guard -> conditioning repeated K times (k-major) -> the sampler at batch K*B.
+// Workspace (floats): vc [n_v] | z_in [n_zi] | cond [K][n_z] | z0 [K][n_z] | flag [2] ints; z0 receives the sampled
+// latents, flag[0] the checkpoints so far, flag[1] the sampler's own guards.
+struct GenFront {
+  float* z0;
+  int* flag;
+};
+static int generate_front(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const float* v_in, const float* z_init,
+                          int K, int B, int T_in, int T_out, int H, int W, size_t extra_bytes, GenFront& g,
+                          cudaStream_t st) {
+  if (u->u.desc.latent_dim != v->v.desc.latent_dim) return fail("generate: U-Net / VAE latent_dim mismatch");
+  const int L = v->v.desc.latent_dim, Cin = v->v.desc.in_channels, h = H / 4, w = W / 4;
+  const size_t n_v = (size_t)B * Cin * T_in * H * W, n_zi = (size_t)B * L * T_in * h * w,
+               n_z = (size_t)B * L * T_out * h * w;
+  if (gen_workspace(u, (n_v + n_zi + 2 * K * n_z) * sizeof(float) + 256 + extra_bytes, st)) return -1;
+  float* vc = u->gen_ws;
+  float* z_in = vc + n_v;
+  float* cond = z_in + n_zi;
+  float* z0 = cond + K * n_z;
+  int* flag = reinterpret_cast<int*>(z0 + K * n_z);
+  B2V_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
+  B2V_CUDA(cudaMemcpyAsync(vc, v_in, n_v * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  launch_guard(vc, (long long)n_v, 0, flag, st);
+  if (v->v.encode(vc, z_in, B, T_in, H, W, st)) return -1;
+  launch_guard(z_in, (long long)n_zi, 1, flag, st);
+  const float* c = z_in;
+  if (T_out != T_in) {
+    launch_upsample_depth(z_in, cond, B * L, T_in, T_out, (long long)h * w, st);
+    launch_guard(cond, (long long)n_z, 1, flag, st);
+    g_launches += 2;
+    c = cond;
+  }
+  if (K > 1) {
+    for (int k = 0; k < K; ++k)
+      if (cond + k * n_z != c)
+        B2V_CUDA(cudaMemcpyAsync(cond + k * n_z, c, n_z * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    c = cond;
+  }
+  const int KB = K * B;
+  if (cfg->sampler == 0) {
+    if (u->u.ddim_sample(z_init, c, z0, KB, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
+                         cfg->n_train, cfg->eta, cfg->noise, flag + 1, st))
+      return -1;
+  } else if (cfg->sampler == 1) {
+    if (u->u.ddpm_sample(z_init, c, z0, KB, T_out, h, w, cfg->ddpm_coef, cfg->n, cfg->noise,
+                         (unsigned long long)cfg->seed, st))
+      return -1;
+  } else if (cfg->sampler == 2 || cfg->sampler == 3) {
+    if (u->u.dpmpp_sample(z_init, c, z0, KB, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
+                          cfg->n_train, 2, cfg->sampler == 3, cfg->noise, flag + 1, st))
+      return -1;
+  }
+  g.z0 = z0;
+  g.flag = flag;
+  return 0;
+}
+
+// *nan_flag = flag[0] | flag[1] (the device-side OR of all checkpoints), when the caller asked for it
+static int report_nan_flag(int* flag, int* nan_flag, cudaStream_t st) {
+  if (!nan_flag) return 0;
+  launch_or_flag(flag, flag + 1, st);
+  g_launches += 1;
+  B2V_CUDA(cudaMemcpyAsync(nan_flag, flag, sizeof(int), cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
 static int write_json(const std::string& js, char* buf, size_t cap) {
   if (js.size() + 1 > cap) return fail("profile: buffer too small (" + std::to_string(js.size() + 1) + " needed)");
   memcpy(buf, js.c_str(), js.size() + 1);
@@ -153,72 +249,61 @@ int b2v_philox_normal(float* out, uint64_t seed, int step, long long n, void* st
 int b2v_generate(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const float* v_in, const float* z_init,
                  float* v_out, int B, int T_in, int T_out, int H, int W, int* nan_flag, void* stream) {
   if (!u || !v || !cfg || !v_in || !z_init || !v_out) return fail("generate: null argument");
-  if (B < 0 || T_in < 1 || T_out < 1 || H < 4 || W < 4 || H % 4 || W % 4) return fail("generate: bad shape");
-  if (cfg->sampler < 0 || cfg->sampler > 3)
-    return fail("generate: unknown sampler (0 = ddim, 1 = ddpm, 2 = dpmpp_2m, 3 = dpmpp_2m_sde)");
-  if (cfg->sampler >= 2) {  // reject a bad DPM-Solver++ configuration before the encoder is launched
-    if (cfg->sampler == 3 && !cfg->noise) return fail("generate: dpmpp_2m_sde needs the per-step noise draws");
-    if (cfg->n < 1 || cfg->n > 4096) return fail("generate: 1 <= n <= 4096 timesteps");
-    std::vector<float> rows((size_t)cfg->n * 8);
-    if (dpmpp_coefficients((const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod, cfg->n_train, 2,
-                           cfg->sampler == 3, rows.data()))
-      return -1;
-  }
+  if (check_generate_args("generate", cfg, B, T_in, T_out, H, W)) return -1;
   if (B == 0) return 0;
-  if (u->u.desc.latent_dim != v->v.desc.latent_dim) return fail("generate: U-Net / VAE latent_dim mismatch");
+  cudaStream_t st = (cudaStream_t)stream;
+  GenFront g;
+  if (generate_front(u, v, cfg, v_in, z_init, 1, B, T_in, T_out, H, W, 0, g, st)) return -1;
+  const int L = v->v.desc.latent_dim, Cin = v->v.desc.in_channels;
+  const size_t n_z = (size_t)B * L * T_out * (H / 4) * (W / 4), n_out = (size_t)B * Cin * T_out * H * W;
+  launch_guard(g.z0, (long long)n_z, 1, g.flag, st);
+  if (v->v.decode(g.z0, v_out, B, T_out, H / 4, W / 4, st)) return -1;
+  launch_guard(v_out, (long long)n_out, 1, g.flag, st);
+  g_launches += 4;
+  if (report_nan_flag(g.flag, nan_flag, st)) return -1;
+  return check_launches("generate");
+}
+
+int b2v_generate_ensemble(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const float* v_in, const float* z_init,
+                          int K, float* members_out, float* mean_out, float* std_out, int B, int T_in, int T_out, int H,
+                          int W, int* nan_flag, void* stream) {
+  if (!u || !v || !cfg || !v_in || !z_init || !mean_out || !std_out) return fail("generate_ensemble: null argument");
+  if (K < 2) return fail("generate_ensemble: K >= 2 samples per input (the std needs two)");
+  if (check_generate_args("generate_ensemble", cfg, B, T_in, T_out, H, W)) return -1;
+  if ((long long)K * B > INT32_MAX) return fail("generate_ensemble: K * B too large");
+  if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int L = v->v.desc.latent_dim, Cin = v->v.desc.in_channels, h = H / 4, w = W / 4;
-  const size_t n_v = (size_t)B * Cin * T_in * H * W, n_zi = (size_t)B * L * T_in * h * w,
-               n_z = (size_t)B * L * T_out * h * w, n_out = (size_t)B * Cin * T_out * H * W;
-  const size_t need = (n_v + n_zi + 2 * n_z) * sizeof(float) + 256;
-  if (need > u->gen_cap) {
-    B2V_CUDA(cudaStreamSynchronize(st));
-    if (u->gen_ws) cudaFree(u->gen_ws);
-    u->gen_ws = nullptr;
-    u->gen_cap = 0;
-    B2V_CUDA(cudaMalloc(&u->gen_ws, need));
-    u->gen_cap = need;
+  const size_t n_z = (size_t)B * L * T_out * h * w, n_out = (size_t)B * Cin * T_out * H * W;
+  // without members_out the decoded members go to the scratch, behind the flags (256-byte aligned)
+  GenFront g;
+  if (generate_front(u, v, cfg, v_in, z_init, K, B, T_in, T_out, H, W, members_out ? 0 : K * n_out * sizeof(float) + 256,
+                     g, st))
+    return -1;
+  float* members = members_out;
+  if (!members) {
+    const uintptr_t p = reinterpret_cast<uintptr_t>(g.flag + 2);
+    members = reinterpret_cast<float*>((p + 255) & ~(uintptr_t)255);
   }
-  float* vc = u->gen_ws;
-  float* z_in = vc + n_v;
-  float* cond = z_in + n_zi;
-  float* z0 = cond + n_z;
-  int* flag = reinterpret_cast<int*>(z0 + n_z);  // [0]: the generate() checkpoints, [1]: the sampler's own guards
-  B2V_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
-  B2V_CUDA(cudaMemcpyAsync(vc, v_in, n_v * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  launch_guard(vc, (long long)n_v, 0, flag, st);
-  if (v->v.encode(vc, z_in, B, T_in, H, W, st)) return -1;
-  launch_guard(z_in, (long long)n_zi, 1, flag, st);
-  const float* c = z_in;
-  if (T_out != T_in) {
-    launch_upsample_depth(z_in, cond, B * L, T_in, T_out, (long long)h * w, st);
-    launch_guard(cond, (long long)n_z, 1, flag, st);
-    g_launches += 2;
-    c = cond;
-  }
-  if (cfg->sampler == 0) {
-    if (u->u.ddim_sample(z_init, c, z0, B, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
-                         cfg->n_train, cfg->eta, cfg->noise, flag + 1, st))
-      return -1;
-  } else if (cfg->sampler == 1) {
-    if (u->u.ddpm_sample(z_init, c, z0, B, T_out, h, w, cfg->ddpm_coef, cfg->n, cfg->noise,
-                         (unsigned long long)cfg->seed, st))
-      return -1;
-  } else if (cfg->sampler == 2 || cfg->sampler == 3) {
-    if (u->u.dpmpp_sample(z_init, c, z0, B, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
-                          cfg->n_train, 2, cfg->sampler == 3, cfg->noise, flag + 1, st))
-      return -1;
-  }
-  launch_guard(z0, (long long)n_z, 1, flag, st);
-  if (v->v.decode(z0, v_out, B, T_out, h, w, st)) return -1;
-  launch_guard(v_out, (long long)n_out, 1, flag, st);
-  g_launches += 4;
-  if (nan_flag) {
-    launch_or_flag(flag, flag + 1, st);
-    g_launches += 1;
-    B2V_CUDA(cudaMemcpyAsync(nan_flag, flag, sizeof(int), cudaMemcpyDeviceToDevice, st));
-  }
-  return check_launches("generate");
+  launch_guard(g.z0, (long long)(K * n_z), 1, g.flag, st);
+  for (int k = 0; k < K; ++k)  // K chunks of B: the batch-B decode program generate() uses
+    if (v->v.decode(g.z0 + k * n_z, members + k * n_out, B, T_out, h, w, st)) return -1;
+  launch_guard(members, (long long)(K * n_out), 1, g.flag, st);
+  launch_ensemble_stats(members, mean_out, std_out, K, (long long)n_out, st);
+  g_launches += 5;  // the four guards and the statistics
+  if (report_nan_flag(g.flag, nan_flag, st)) return -1;
+  return check_launches("generate_ensemble");
+}
+
+int b2v_ensemble_stats(const float* members, float* mean, float* stdev, int K, long long n, void* stream) {
+  if (!members || !mean || !stdev) return fail("ensemble_stats: null argument");
+  if (K < 2) return fail("ensemble_stats: K >= 2 members (the std needs two)");
+  if (n < 0) return fail("ensemble_stats: negative n");
+  if (check_device()) return -1;
+  if (n == 0) return 0;
+  launch_ensemble_stats(members, mean, stdev, K, n, (cudaStream_t)stream);
+  g_launches += 1;
+  return check_launches("ensemble_stats");
 }
 
 int b2v_q_sample(const float* z0, const float* noise, const int64_t* t, const float* sqrt_ac, const float* sqrt_1m_ac,

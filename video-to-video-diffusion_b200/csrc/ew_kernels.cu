@@ -1162,7 +1162,7 @@ __global__ void stitch_accumulate_kernel(const float* __restrict__ patch, float*
     const float wt = __fmul_rn(__fmul_rn(gd[d], gh[h]), gw[w]);  // the reference's outer-product order
     const size_t o = ((size_t)bc * D + (d0 + d)) * H * W + (size_t)(h0 + h) * W + (w0 + w);
     acc[o] = __fadd_rn(acc[o], __fmul_rn(patch[i], wt));
-    wsum[o] = __fadd_rn(wsum[o], wt);
+    if (wsum) wsum[o] = __fadd_rn(wsum[o], wt);  // null: a second quantity blended with weights summed elsewhere
   }
 }
 void launch_stitch_accumulate(const float* patch, float* acc, float* wsum, const float* gd, const float* gh,
@@ -1184,6 +1184,67 @@ void launch_stitch_normalize(float* acc, const float* wsum, long long n, cudaStr
   int blocks = cdiv(n, 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
   launch_k(stitch_normalize_kernel, dim3(blocks), dim3(256), 0, st, acc, wsum, n);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Ensemble statistics: per voxel i of K decoded samples members[k][i] (k-major),
+//   mean = sum_k x / K,  std = sqrt(max(0, (sum_k x^2 - sum_k x * mean) / (K - 1)))   (unbiased, like torch.std)
+// Both sums are fp64 registers over k = 0..K-1 in order; one thread owns a voxel (no atomics, no cross-thread
+// reduction), so the result is bitwise reproducible.  HBM-bound: K*4 + 8 bytes per voxel.  With n % 4 == 0 and
+// 16-byte aligned pointers every row is read in 16-byte vectors; otherwise element by element (same arithmetic).
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void ensemble_voxel(double s, double q, int K, float& mean, float& sd) {
+  const double m = s / K;
+  const double var = (q - s * m) / (K - 1);
+  mean = (float)m;
+  sd = (float)sqrt(var > 0.0 ? var : 0.0);
+}
+__global__ void __launch_bounds__(256) ensemble_stats_kernel(const float* __restrict__ members, float* __restrict__ mean,
+                                                             float* __restrict__ sd, int K, long long n, int vec) {
+  pdl_trigger();
+  pdl_wait();
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  if (vec) {
+    const float4* m4 = reinterpret_cast<const float4*>(members);
+    const long long n4 = n / 4;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+      double s[4] = {0.0, 0.0, 0.0, 0.0}, q[4] = {0.0, 0.0, 0.0, 0.0};
+#pragma unroll 4
+      for (int k = 0; k < K; ++k) {
+        const float4 x = __ldcs(m4 + (size_t)k * n4 + i);  // read once: do not keep it in L2
+        const float xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          s[j] += (double)xs[j];
+          q[j] = fma((double)xs[j], (double)xs[j], q[j]);
+        }
+      }
+      float4 mo, so;
+      ensemble_voxel(s[0], q[0], K, mo.x, so.x);
+      ensemble_voxel(s[1], q[1], K, mo.y, so.y);
+      ensemble_voxel(s[2], q[2], K, mo.z, so.z);
+      ensemble_voxel(s[3], q[3], K, mo.w, so.w);
+      reinterpret_cast<float4*>(mean)[i] = mo;
+      reinterpret_cast<float4*>(sd)[i] = so;
+    }
+    return;
+  }
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    double s = 0.0, q = 0.0;
+    for (int k = 0; k < K; ++k) {
+      const double x = (double)members[(size_t)k * n + i];
+      s += x;
+      q = fma(x, x, q);
+    }
+    ensemble_voxel(s, q, K, mean[i], sd[i]);
+  }
+}
+void launch_ensemble_stats(const float* members, float* mean, float* sd, int K, long long n, cudaStream_t st) {
+  const bool vec = n % 4 == 0 && ((uintptr_t)members | (uintptr_t)mean | (uintptr_t)sd) % 16 == 0;
+  int blocks = cdiv(vec ? n / 4 : n, 256);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks < 1) blocks = 1;
+  launch_k(ensemble_stats_kernel, dim3(blocks), dim3(256), 0, st, members, mean, sd, K, n, (int)vec);
 }
 
 // ------------------------------------------------------------------------------------------------

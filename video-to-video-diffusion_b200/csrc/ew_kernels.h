@@ -68,6 +68,8 @@ void launch_stitch_accumulate(const float* patch, float* acc, float* wsum, const
                               const float* gw, int BC, int pd, int ph, int pw, int D, int H, int W, int d0, int h0,
                               int w0, cudaStream_t st);
 void launch_stitch_normalize(float* acc, const float* wsum, long long n, cudaStream_t st);
+// per-voxel mean and unbiased std of K members [K][n] (fp64 accumulation in k order; see ew_kernels.cu)
+void launch_ensemble_stats(const float* members, float* mean, float* sd, int K, long long n, cudaStream_t st);
 size_t video_metrics_ws_bytes(int BC, int T, int H, int W);
 void launch_video_metrics(const float* a, const float* b, float* out, float* ws, int BC, int T, int H, int W,
                           float max_val, cudaStream_t st);

@@ -172,7 +172,8 @@ def gaussian_window_1d(n, device):
 
 
 def stitch_accumulate(patch, acc, wsum, d0, h0, w0, win=None):
-    """acc[..., d0:d0+pd, h0:h0+ph, w0:w0+pw] += patch * window ; wsum likewise (in place, fp32 NCDHW)"""
+    """acc[..., d0:d0+pd, h0:h0+ph, w0:w0+pw] += patch * window ; wsum likewise (in place, fp32 NCDHW); wsum None
+    writes acc only (a second quantity blended with the weights another call sums)"""
     B, C, pd, ph, pw = patch.shape
     _, _, D, H, W = acc.shape
     gd, gh, gw = win if win is not None else (gaussian_window_1d(pd, patch.device), gaussian_window_1d(ph, patch.device),
@@ -180,6 +181,22 @@ def stitch_accumulate(patch, acc, wsum, d0, h0, w0, win=None):
     _lib.check(_lib.lib().b2v_stitch_accumulate(_lib.dptr(patch.contiguous()), _lib.dptr(acc), _lib.dptr(wsum),
                                                 _lib.dptr(gd), _lib.dptr(gh), _lib.dptr(gw), B * C, pd, ph, pw, D, H, W,
                                                 int(d0), int(h0), int(w0), _lib.stream()), "stitch_accumulate")
+
+
+def ensemble_stats(members):
+    """members (K, ...) fp32 CUDA, K >= 2 -> (mean, std) of shape members.shape[1:]: the per-element mean and unbiased
+    standard deviation over the K members, accumulated in fp64 in member order (bitwise reproducible)"""
+    if members.dim() < 1 or members.shape[0] < 2:
+        raise ValueError(f"ensemble_stats: need K >= 2 members along dim 0, got shape {tuple(members.shape)}")
+    members = members.contiguous()
+    mean = torch.empty(members.shape[1:], dtype=torch.float32, device=members.device)
+    std = torch.empty_like(mean)
+    if mean.numel() == 0:
+        return mean, std
+    with torch.cuda.device(members.device):
+        _lib.check(_lib.lib().b2v_ensemble_stats(_lib.dptr(members), _lib.dptr(mean), _lib.dptr(std), members.shape[0],
+                                                 mean.numel(), _lib.stream()), "ensemble_stats")
+    return mean, std
 
 
 def stitch_normalize(acc, wsum):
