@@ -123,6 +123,32 @@ int b2v_dpmpp_sample(b2v_unet* u, const float* z_init, const float* cond, float*
                      const float* noise, int* nan_flag, void* stream);
 int b2v_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* noise, const float* coef, long long n,
                      int* nan_flag, void* stream);
+/* UniPC (Zhao et al. 2023, "UniPC: A Unified Predictor-Corrector Framework for Fast Sampling of Diffusion Models"),
+ * data prediction over the eps-prediction U-Net, without guidance; not in the reference.  One U-Net evaluation per
+ * step: the corrector UniC reuses the evaluation the next predictor needs.  alpha, sigma, lambda, the timesteps and the
+ * last step to the clean sample are as for DPM-Solver++.  m_i = clamp((z_i - sigma_i eps_i) / alpha_i, +-10) is the
+ * data prediction at the evaluated (uncorrected) state.  Step i:
+ *   corrector (i >= 1, order of the previous predictor): xc_i = g z_i + a_c xc_{i-1} + sum_{j=0..3} c_j m_{i-j}
+ *   predictor, order k_i = min(order, i+1, n-i):          z_{i+1} = a_p xc_i + sum_{j=0..2} p_j m_{i-j}
+ *   (xc_0 = z_0: g = 1, a_c = 0 at step 0; the last step gives z = m_{n-1}).  variant 0 = bh1: B(h) = -h,
+ *   1 = bh2: B(h) = expm1(-h).  With the corrector off, order 1 and order 2 with bh2 are DPM-Solver++(2M).
+ * b2v_unipc_coefficients writes the rows {sigma_i, alpha_i, g, a_c, c0, c1, c2, c3, a_p, p0, p1, p2, clip = 10, 0, 0, 0}
+ *   (HOST fp32 [n][16], computed in fp64).  HOST only, needs no device.  Fails for n outside [1, 4096], order not 1..3,
+ *   variant not 0 or 1, timesteps not strictly decreasing or outside [0, n_train), an alphas_cumprod entry outside
+ *   (0, 1), or a null pointer.
+ * b2v_unipc_sample: the whole loop, one CUDA-graph replay per step (U-Net + update), no host synchronisation;
+ *   timesteps / alphas_cumprod / nan_flag as in b2v_dpmpp_sample.
+ * b2v_unipc_update: step `step` (>= 0) of a loop, in place: reads z (the evaluated state), eps, and xc / hist only where
+ *   the row's weights are non-zero; writes z (the next state), xc (the corrected state) and m_step into slot step % 4 of
+ *   hist (DEVICE fp32 [4][n], the data-prediction ring; m_{step-j} is read from slot (step - j) % 4).  coef = DEVICE
+ *   fp32[16], one row.  *nan_flag (DEVICE int, may be NULL) is set when a NaN/Inf guard fired.                      */
+int b2v_unipc_coefficients(const int64_t* timesteps, int n, const float* alphas_cumprod, int n_train, int order,
+                           int variant, float* rows);
+int b2v_unipc_sample(b2v_unet* u, const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                     const int64_t* timesteps, int n, const float* alphas_cumprod, int n_train, int order, int variant,
+                     int* nan_flag, void* stream);
+int b2v_unipc_update(float* z, float* xc, float* hist, const float* eps, const float* coef, int step, long long n,
+                     int* nan_flag, void* stream);
 /* inference/sampler.py:221-239  DDIMSampler._get_timesteps: every (n_train // steps)-th timestep plus n_train-1 if
  * missing, descending; writes at most cap entries to HOST out and returns the count (steps or steps + 1), <0 on error */
 int b2v_ddim_timesteps(int n_train, int num_inference_steps, int64_t* out, int cap);
@@ -157,15 +183,18 @@ int b2v_vae_decode(b2v_vae* v, const float* z, float* x, int B, int T, int h, in
  * The schedule is passed as host tables so that the caller's GaussianDiffusion buffers are the single source.      */
 typedef struct {
   int sampler;                 /* 0 = DDIM (b2v_ddim_sample), 1 = DDPM (b2v_ddpm_sample), 2 = DPM-Solver++(2M),
-                                  3 = DPM-Solver++(2M) SDE (b2v_dpmpp_sample, order 2; 3 needs `noise`) */
-  int n;                       /* DDIM / DPM-Solver++: entries of `timesteps`; DDPM: number of training timesteps */
-  const int64_t* timesteps;    /* DDIM / DPM-Solver++: HOST int64[n] */
-  const float* alphas_cumprod; /* DDIM / DPM-Solver++: HOST fp32[n_train] */
+                                  3 = DPM-Solver++(2M) SDE (b2v_dpmpp_sample, order 2; 3 needs `noise`),
+                                  4 = UniPC (b2v_unipc_sample, with unipc_order and unipc_variant) */
+  int n;                       /* DDIM / DPM-Solver++ / UniPC: entries of `timesteps`; DDPM: training timesteps */
+  const int64_t* timesteps;    /* DDIM / DPM-Solver++ / UniPC: HOST int64[n] */
+  const float* alphas_cumprod; /* DDIM / DPM-Solver++ / UniPC: HOST fp32[n_train] */
   int n_train;
   float eta;                   /* DDIM */
   const float* ddpm_coef;      /* DDPM: HOST fp32 [n][8] */
   const float* noise;          /* DEVICE per-step draws [n][numel(z)] or NULL (see b2v_ddim_sample / b2v_ddpm_sample) */
   uint64_t seed;               /* DDPM with noise == NULL */
+  int unipc_order;             /* UniPC: 1, 2 or 3 (read only when sampler == 4) */
+  int unipc_variant;           /* UniPC: 0 = bh1, 1 = bh2 (read only when sampler == 4) */
 } b2v_sampler_cfg;
 int b2v_generate(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, const float* v_in, const float* z_init,
                  float* v_out, int B, int T_in, int T_out, int H, int W, int* nan_flag, void* stream);

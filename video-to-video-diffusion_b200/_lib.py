@@ -35,7 +35,7 @@ class SamplerCfg(ctypes.Structure):
     """b2v_sampler_cfg: the schedule tables b2v_generate runs its sampler with (host pointers; noise is a device pointer)"""
     _fields_ = [("sampler", c_int), ("n", c_int), ("timesteps", POINTER(c_int64)), ("alphas_cumprod", POINTER(c_float)),
                 ("n_train", c_int), ("eta", c_float), ("ddpm_coef", POINTER(c_float)), ("noise", c_void_p),
-                ("seed", c_uint64)]
+                ("seed", c_uint64), ("unipc_order", c_int), ("unipc_variant", c_int)]
 
 
 # name -> (restype, argtypes); mirrors include/b2v.h one to one
@@ -56,6 +56,10 @@ SIGNATURES = {
     "b2v_dpmpp_sample": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, POINTER(c_int64), c_int, POINTER(c_float),
                                  c_int, c_int, c_int, _P, _P, _P]),
     "b2v_dpmpp_update": (c_int, [_P, _P, _P, _P, _P, c_longlong, _P, _P]),
+    "b2v_unipc_coefficients": (c_int, [POINTER(c_int64), c_int, POINTER(c_float), c_int, c_int, c_int, POINTER(c_float)]),
+    "b2v_unipc_sample": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, POINTER(c_int64), c_int, POINTER(c_float),
+                                 c_int, c_int, c_int, _P, _P]),
+    "b2v_unipc_update": (c_int, [_P, _P, _P, _P, _P, c_int, c_longlong, _P, _P]),
     "b2v_sampler_begin": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, _P]),
     "b2v_ddpm_step": (c_int, [_P, c_int64, POINTER(c_float), _P, _P]),
     "b2v_sampler_end": (c_int, [_P, _P, _P]),

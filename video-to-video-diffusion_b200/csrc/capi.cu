@@ -53,9 +53,15 @@ static int store_weight(WeightMap& wm, bool finalized, const char* key, const fl
 static int check_generate_args(const std::string& who, const b2v_sampler_cfg* cfg, int B, int T_in, int T_out, int H,
                                int W) {
   if (B < 0 || T_in < 1 || T_out < 1 || H < 4 || W < 4 || H % 4 || W % 4) return fail(who + ": bad shape");
-  if (cfg->sampler < 0 || cfg->sampler > 3)
-    return fail(who + ": unknown sampler (0 = ddim, 1 = ddpm, 2 = dpmpp_2m, 3 = dpmpp_2m_sde)");
-  if (cfg->sampler >= 2) {  // reject a bad DPM-Solver++ configuration before the encoder is launched
+  if (cfg->sampler < 0 || cfg->sampler > 4)
+    return fail(who + ": unknown sampler (0 = ddim, 1 = ddpm, 2 = dpmpp_2m, 3 = dpmpp_2m_sde, 4 = unipc)");
+  if (cfg->sampler == 4) {  // reject a bad UniPC configuration (tables, order, variant) before the encoder is launched
+    if (cfg->n < 1 || cfg->n > 4096) return fail(who + ": 1 <= n <= 4096 timesteps");
+    std::vector<float> rows((size_t)cfg->n * 16);
+    if (unipc_coefficients((const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod, cfg->n_train,
+                           cfg->unipc_order, cfg->unipc_variant, rows.data()))
+      return -1;
+  } else if (cfg->sampler >= 2) {  // reject a bad DPM-Solver++ configuration before the encoder is launched
     if (cfg->sampler == 3 && !cfg->noise) return fail(who + ": dpmpp_2m_sde needs the per-step noise draws");
     if (cfg->n < 1 || cfg->n > 4096) return fail(who + ": 1 <= n <= 4096 timesteps");
     std::vector<float> rows((size_t)cfg->n * 8);
@@ -130,6 +136,10 @@ static int generate_front(b2v_unet* u, b2v_vae* v, const b2v_sampler_cfg* cfg, c
     if (u->u.dpmpp_sample(z_init, c, z0, KB, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
                           cfg->n_train, 2, cfg->sampler == 3, cfg->noise, flag + 1, st))
       return -1;
+  } else if (cfg->sampler == 4) {
+    if (u->u.unipc_sample(z_init, c, z0, KB, T_out, h, w, (const long long*)cfg->timesteps, cfg->n, cfg->alphas_cumprod,
+                          cfg->n_train, cfg->unipc_order, cfg->unipc_variant, flag + 1, st))
+      return -1;
   }
   g.z0 = z0;
   g.flag = flag;
@@ -203,6 +213,17 @@ int b2v_dpmpp_sample(b2v_unet* u, const float* z_init, const float* cond, float*
   if (!u) return fail("dpmpp_sample: null handle");
   return u->u.dpmpp_sample(z_init, cond, z_out, B, T, h, w, (const long long*)timesteps, n, alphas_cumprod, n_train,
                            order, sde, noise, nan_flag, (cudaStream_t)stream);
+}
+int b2v_unipc_coefficients(const int64_t* timesteps, int n, const float* alphas_cumprod, int n_train, int order,
+                           int variant, float* rows) {
+  return unipc_coefficients((const long long*)timesteps, n, alphas_cumprod, n_train, order, variant, rows);
+}
+int b2v_unipc_sample(b2v_unet* u, const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                     const int64_t* timesteps, int n, const float* alphas_cumprod, int n_train, int order, int variant,
+                     int* nan_flag, void* stream) {
+  if (!u) return fail("unipc_sample: null handle");
+  return u->u.unipc_sample(z_init, cond, z_out, B, T, h, w, (const long long*)timesteps, n, alphas_cumprod, n_train,
+                           order, variant, nan_flag, (cudaStream_t)stream);
 }
 int b2v_sampler_begin(b2v_unet* u, const float* z_init, const float* cond, int B, int T, int h, int w, void* stream) {
   if (!u) return fail("sampler_begin: null handle");
@@ -579,6 +600,15 @@ int b2v_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* no
   launch_dpmpp_update(z, x0_prev, eps, noise, coef, nullptr, n, nan_flag, (cudaStream_t)stream);
   g_launches += 1;
   return check_launches("dpmpp_update");
+}
+int b2v_unipc_update(float* z, float* xc, float* hist, const float* eps, const float* coef, int step, long long n,
+                     int* nan_flag, void* stream) {
+  if (!z || !xc || !hist || !eps || !coef) return fail("unipc_update: null argument");
+  if (step < 0) return fail("unipc_update: negative step");
+  if (n <= 0) return 0;
+  launch_unipc_update(z, xc, hist, eps, coef, nullptr, step, n, nan_flag, (cudaStream_t)stream);
+  g_launches += 1;
+  return check_launches("unipc_update");
 }
 
 }  // extern "C"

@@ -715,6 +715,82 @@ __global__ void dpmpp_update_kernel(float* z, float* x0_prev, const float* __res
   if (flag && nan_flag) atomicOr(nan_flag, 1);
 }
 
+// UniPC predictor-corrector update (Zhao et al. 2023, data prediction; see b2v_unipc_coefficients for the rows), in
+// this fp32 order so that a torch eager chain reproduces it bit for bit:
+//   row = {sigma, alpha, g, a_c, c0, c1, c2, c3, a_p, p0, p1, p2, clip, 0, 0, 0}
+//   m  = clamp(guard((z - sigma*e) / alpha), +-clip)                       (e = guard(eps))
+//   xc = guard(0 + g*z + a_c*xc_prev + c0*m + c1*m_1 + c2*m_2 + c3*m_3)   (corrector)
+//   z  = guard(0 + a_p*xc + p0*m + p1*m_1 + p2*m_2)                        (predictor)
+// left to right, a term whose weight is 0 skipped (its operand is not read, so an unwritten slot or xc_prev cannot
+// leak into the result, NaN or not).  m_j is the data prediction of step - j, slot (step - j) % 4 of hist [4][n]; m
+// goes to slot step % 4 and xc replaces xc_prev.
+struct UniRow {
+  float sig, alp, g, ac, c0, c1, c2, c3, ap, p0, p1, p2, clip;
+};
+__device__ __forceinline__ float uni_term(float acc, float w, float v) {
+  return w != 0.f ? __fadd_rn(acc, __fmul_rn(w, v)) : acc;
+}
+__device__ __forceinline__ void unipc_one(const UniRow& r, float z, float e, float xp, float m1, float m2, float m3,
+                                          float& zo, float& xo, float& mo, int* flag) {
+  e = nan_guard(e, flag);
+  float m = nan_guard(__fdiv_rn(__fsub_rn(z, __fmul_rn(r.sig, e)), r.alp), flag);
+  m = fminf(fmaxf(m, -r.clip), r.clip);
+  float x = uni_term(0.f, r.g, z);
+  x = uni_term(x, r.ac, xp);
+  x = uni_term(x, r.c0, m);
+  x = uni_term(x, r.c1, m1);
+  x = uni_term(x, r.c2, m2);
+  x = nan_guard(uni_term(x, r.c3, m3), flag);
+  float zn = uni_term(0.f, r.ap, x);
+  zn = uni_term(zn, r.p0, m);
+  zn = uni_term(zn, r.p1, m1);
+  zn = nan_guard(uni_term(zn, r.p2, m2), flag);
+  zo = zn;
+  xo = x;
+  mo = m;
+}
+__global__ void __launch_bounds__(256) unipc_update_kernel(float* z, float* xc, float* hist, const float* __restrict__ eps,
+                                                           const float* __restrict__ coef_table,
+                                                           const SamplerCtl* __restrict__ ctl, int step_imm, long long n,
+                                                           int* nan_flag, int vec) {
+  pdl_trigger();
+  pdl_wait();
+  const int step = ctl ? ctl->step : step_imm;
+  const float* c = coef_table + (ctl ? (size_t)step * 16 : 0);
+  const UniRow r{c[0], c[1], c[2], c[3], c[4], c[5], c[6], c[7], c[8], c[9], c[10], c[11], c[12]};
+  float* m0p = hist + (size_t)(step & 3) * n;
+  const float* m1p = hist + (size_t)((step + 3) & 3) * n;
+  const float* m2p = hist + (size_t)((step + 2) & 3) * n;
+  const float* m3p = hist + (size_t)((step + 1) & 3) * n;
+  const bool rx = r.ac != 0.f, r1 = r.c1 != 0.f || r.p1 != 0.f, r2 = r.c2 != 0.f || r.p2 != 0.f, r3 = r.c3 != 0.f;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  int flag = 0;
+  if (vec) {
+    const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n / 4; i += stride) {
+      const float4 zv = reinterpret_cast<const float4*>(z)[i];
+      const float4 ev = __ldcs(reinterpret_cast<const float4*>(eps) + i);
+      const float4 xv = rx ? reinterpret_cast<const float4*>(xc)[i] : zero4;
+      const float4 a1 = r1 ? reinterpret_cast<const float4*>(m1p)[i] : zero4;
+      const float4 a2 = r2 ? reinterpret_cast<const float4*>(m2p)[i] : zero4;
+      const float4 a3 = r3 ? reinterpret_cast<const float4*>(m3p)[i] : zero4;
+      float4 zo, xo, mo;
+      unipc_one(r, zv.x, ev.x, xv.x, a1.x, a2.x, a3.x, zo.x, xo.x, mo.x, &flag);
+      unipc_one(r, zv.y, ev.y, xv.y, a1.y, a2.y, a3.y, zo.y, xo.y, mo.y, &flag);
+      unipc_one(r, zv.z, ev.z, xv.z, a1.z, a2.z, a3.z, zo.z, xo.z, mo.z, &flag);
+      unipc_one(r, zv.w, ev.w, xv.w, a1.w, a2.w, a3.w, zo.w, xo.w, mo.w, &flag);
+      reinterpret_cast<float4*>(z)[i] = zo;
+      reinterpret_cast<float4*>(xc)[i] = xo;
+      reinterpret_cast<float4*>(m0p)[i] = mo;
+    }
+  } else {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      unipc_one(r, z[i], eps[i], rx ? xc[i] : 0.f, r1 ? m1p[i] : 0.f, r2 ? m2p[i] : 0.f, r3 ? m3p[i] : 0.f, z[i], xc[i],
+                m0p[i], &flag);
+  }
+  if (flag && nan_flag) atomicOr(nan_flag, 1);
+}
+
 // Philox4x32-10 (Salmon et al., SC'11; the counter-based generator behind cuRAND / torch CUDA): counter
 // (c0..c3), key (k0, k1) -> four 32-bit words.  Used for the DDPM ancestral noise when the caller passes none.
 __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
@@ -811,6 +887,16 @@ void launch_dpmpp_update(float* z, float* x0_prev, const float* eps, const float
   int blocks = cdiv(n, 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
   launch_k(dpmpp_update_kernel, dim3(blocks), dim3(256), 0, st, z, x0_prev, eps, noise, coef_table, ctl, n, nan_flag);
+}
+void launch_unipc_update(float* z, float* xc, float* hist, const float* eps, const float* coef_table,
+                         const SamplerCtl* ctl, int step, long long n, int* nan_flag, cudaStream_t st) {
+  // 16-byte accesses when every row (z, eps, xc and the four hist slots, n floats apart) is 16-byte aligned
+  const bool vec = n % 4 == 0 && ((uintptr_t)z | (uintptr_t)xc | (uintptr_t)hist | (uintptr_t)eps) % 16 == 0;
+  int blocks = cdiv(vec ? n / 4 : n, 256);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks < 1) blocks = 1;
+  launch_k(unipc_update_kernel, dim3(blocks), dim3(256), 0, st, z, xc, hist, eps, coef_table, ctl, step, n, nan_flag,
+           (int)vec);
 }
 void launch_ddpm_update(float* z, const float* eps, const float* noise, const float* coef_table, const SamplerCtl* ctl,
                         const Coef8& coef, long long n, cudaStream_t st) {

@@ -43,6 +43,10 @@ void launch_ddpm_update(float* z, const float* eps, const float* noise, const fl
 // DPM-Solver++(2M) step: row `step` of coef_table (ctl != null) or coef_table[0..7] with immediate noise (ctl == null)
 void launch_dpmpp_update(float* z, float* x0_prev, const float* eps, const float* noise, const float* coef_table,
                          const SamplerCtl* ctl, long long n, int* nan_flag, cudaStream_t st);
+// UniPC step on z, xc and the data-prediction ring hist [4][n]: row `ctl->step` of the [n][16] coef_table (ctl != null)
+// or the single row coef_table[0..15] at loop index `step` (ctl == null)
+void launch_unipc_update(float* z, float* xc, float* hist, const float* eps, const float* coef_table,
+                         const SamplerCtl* ctl, int step, long long n, int* nan_flag, cudaStream_t st);
 void launch_philox_fill(float* out, unsigned long long seed, int step, long long n, cudaStream_t st);
 void launch_guard(float* x, long long n, int mode, int* flag, cudaStream_t st);
 void launch_or_flag(int* dst, const int* src, cudaStream_t st);  // *dst |= *src

@@ -6,6 +6,9 @@
 #include <stddef.h>
 #include <stdlib.h>
 
+#include <algorithm>
+#include <utility>
+
 namespace b2v {
 
 // ------------------------------------------------------------------ weights
@@ -378,7 +381,8 @@ static Op loop_update_op(UProgram& up, int kind) {
   SamplerCtl* ctl = up.ctl;
   int* nf = up.nan_dev;
   const long long numel = up.numel;
-  UProgram* upp = &up;  // x0_prev is allocated by the first dpmpp_sample (before its graph is captured): read at launch
+  UProgram* upp = &up;  // x0_prev / the UniPC buffers: allocated by their sampler's first run (before its graph is
+                        // captured), read at launch
   Op op;
   op.launches = 2;
   switch (kind) {
@@ -396,6 +400,13 @@ static Op loop_update_op(UProgram& up, int kind) {
       op.name = "dpmpp_update";
       op.bytes = (double)numel * 20.0;  // z, eps, x0_prev read; z, x0_prev written (+4 B noise in the SDE form)
       op.run = [=](cudaStream_t st) { launch_dpmpp_update(z, upp->x0_prev, e, nullptr, ct, ctl, numel, nf, st); };
+      break;
+    case SAMPLER_UNIPC:
+      op.name = "unipc_update";
+      op.bytes = (double)numel * 36.0;  // order 3: z, eps, xc_prev, three history slots read; z, xc, m written
+      op.run = [=](cudaStream_t st) {
+        launch_unipc_update(z, upp->unipc_xc, upp->unipc_hist, e, ct, ctl, 0, numel, nf, st);
+      };
       break;
   }
   const auto update = std::move(op.run);
@@ -421,7 +432,7 @@ static int build_unet_program(UNet& u, UProgram& up) {
   up.step_dev = up.ctl ? &up.ctl->step : nullptr;
   up.nan_dev = up.ctl ? &up.ctl->nan_flag : nullptr;
   up.t_table = (long long*)up.ds.alloc(sizeof(long long) * 4096);
-  up.coef_table = (float*)up.ds.alloc(sizeof(float) * 8 * 4096);
+  up.coef_table = (float*)up.ds.alloc(sizeof(float) * 16 * 4096);  // 4096 rows of up to 16 floats
   up.stats_cap = (size_t)B * 64 * 256;
   up.stats = (stat_t*)up.ds.alloc(up.stats_cap * sizeof(stat_t));
   up.silu_temb = (float*)up.ds.alloc((size_t)B * d.time_embed_dim * 4);
@@ -643,14 +654,14 @@ static int temb_tables(const UNet& u, UProgram* up, int n, cudaStream_t st) {
   return 0;
 }
 
-// the loop driver shared by the samplers.  loop_tables: upload a loop's timesteps and [n][8] coefficient rows (loop
-// order) and build its time embedding.
+// the loop driver shared by the samplers.  loop_tables: upload a loop's timesteps and [n][width] coefficient rows
+// (loop order; width 8, or 16 for UniPC) and build its time embedding.
 static int loop_tables(const UNet& u, UProgram* up, const std::vector<long long>& ts, const std::vector<float>& rows,
-                       cudaStream_t st) {
+                       int width, cudaStream_t st) {
   const int n = (int)ts.size();
   // pageable-host copies are staged by the runtime before returning, so the vectors may go out of scope
   B2V_CUDA(cudaMemcpyAsync(up->t_table, ts.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, st));
-  B2V_CUDA(cudaMemcpyAsync(up->coef_table, rows.data(), sizeof(float) * 8 * n, cudaMemcpyHostToDevice, st));
+  B2V_CUDA(cudaMemcpyAsync(up->coef_table, rows.data(), sizeof(float) * width * n, cudaMemcpyHostToDevice, st));
   return temb_tables(u, up, n, st);
 }
 
@@ -700,7 +711,7 @@ int UNet::ddim_sample(const float* z_init, const float* cond, float* z_out, int 
   if (ddim_coefficients(timesteps, n, ac, n_train, eta, coef.data())) return -1;
   if (sampler_begin(z_init, cond, B, T, h, w, st)) return -1;
   UProgram* up = active;
-  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, st)) return -1;
+  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, 8, st)) return -1;
   // the update reads the noise whenever it has a pointer: only the stochastic variant gets step i's draw (row i)
   if (loop_replay(*this, up, SAMPLER_DDIM, 0, n, eta > 0.f ? noise : nullptr, 0, st)) return -1;
   B2V_CUDA(cudaMemcpyAsync(z_out, up->x_in, up->numel * 4, cudaMemcpyDeviceToDevice, st));
@@ -773,12 +784,147 @@ int UNet::dpmpp_sample(const float* z_init, const float* cond, float* z_out, int
     up->x0_prev = (float*)up->ds.alloc(up->numel * 4);
     if (!up->x0_prev) return fail("out of device memory (DPM-Solver++ x0 buffer)");
   }
-  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, st)) return -1;
+  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, 8, st)) return -1;
   // step i's draw is row i of the caller's buffer (the last row is not read: its c is 0)
   if (loop_replay(*this, up, SAMPLER_DPMPP, 0, n, sde ? noise : nullptr, 0, st)) return -1;
   B2V_CUDA(cudaMemcpyAsync(z_out, up->x_in, up->numel * 4, cudaMemcpyDeviceToDevice, st));
   if (nan_flag) B2V_CUDA(cudaMemcpyAsync(nan_flag, up->nan_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
   return check_launches("dpmpp_sample");
+}
+
+// UniPC's h-dependent terms (diffusers multistep_uni_p/c_bh_update with predict_x0): hh = -h, phi1 = expm1(hh),
+// B(h) = hh (bh1) or expm1(hh) (bh2), and b_q = h phi_{q+1}(-h) q! / B(h) for q = 1..k by the phi recursion
+static void unipc_phi(double h, int variant, int k, double& phi1, double& Bh, double* b) {
+  const double hh = -h;
+  phi1 = expm1(hh);
+  Bh = variant == 0 ? hh : expm1(hh);
+  double hphi = phi1 / hh - 1.0, fac = 1.0;
+  for (int q = 1; q <= k; ++q) {
+    b[q - 1] = hphi * fac / Bh;
+    fac *= q + 1;
+    hphi = hphi / hh - 1.0 / fac;
+  }
+}
+
+// rho of the k x k system R rho = b, R[q][j] = r_j^q (k <= 3), Gaussian elimination with partial pivoting
+static void unipc_solve(const double* r, const double* b, int k, double* rho) {
+  double A[3][4];
+  for (int q = 0; q < k; ++q) {
+    for (int j = 0; j < k; ++j) A[q][j] = pow(r[j], q);
+    A[q][k] = b[q];
+  }
+  for (int c = 0; c < k; ++c) {
+    int piv = c;
+    for (int q = c + 1; q < k; ++q)
+      if (fabs(A[q][c]) > fabs(A[piv][c])) piv = q;
+    for (int j = 0; j <= k; ++j) std::swap(A[c][j], A[piv][j]);
+    for (int q = c + 1; q < k; ++q) {
+      const double f = A[q][c] / A[c][c];
+      for (int j = c; j <= k; ++j) A[q][j] -= f * A[c][j];
+    }
+  }
+  for (int c = k - 1; c >= 0; --c) {
+    double s = A[c][k];
+    for (int j = c + 1; j < k; ++j) s -= A[c][j] * rho[j];
+    rho[c] = s / A[c][c];
+  }
+}
+
+// UniPC (Zhao et al. 2023) rows {sigma_i, alpha_i, g, a_c, c0..c3, a_p, p0..p2, clip = 10, 0, 0, 0} in fp64 from the
+// fp32 schedule (alpha, sigma, lambda as for DPM-Solver++).  Step i: the corrector UniC of order k_{i-1} (none at i = 0:
+// g = 1) gives xc = g z + a_c xc_prev + sum_j c_j m_{i-j}; the predictor UniP of order k_i = min(p, i+1, n-i) gives
+// z' = a_p xc + sum_j p_j m_{i-j}, the last step z' = m_{n-1}.  With D_j = (m_{s-j} - m_s) / r_j,
+// r_j = (lambda_{s-j} - lambda_s) / h around the step's base s:
+//   UniC (s = i-1, h = lambda_i - lambda_{i-1}): xc = (sigma_i / sigma_{i-1}) xc_prev - alpha_i phi1 m_{i-1}
+//        - alpha_i B(h) (sum_{j<k} rho_j D_j + rho_k (m_i - m_{i-1})),  R rho = b over r = (r_1 .. r_{k-1}, 1), rho = 0.5 at k = 1
+//   UniP (s = i, h = lambda_{i+1} - lambda_i):   z' = (sigma_{i+1} / sigma_i) xc - alpha_{i+1} phi1 m_i
+//        - alpha_{i+1} B(h) sum_{j<k} rho_j D_j,  rho = 0.5 at k = 2, the leading (k-1) x (k-1) system at k = 3
+int unipc_coefficients(const long long* ts, int n, const float* ac, int n_train, int order, int variant, float* rows) {
+  if (!ts || !ac || !rows) return fail("unipc_coefficients: null argument");
+  if (n < 1 || n > 4096) return fail("unipc_coefficients: 1 <= n <= 4096 timesteps");
+  if (order < 1 || order > 3) return fail("unipc_coefficients: order must be 1, 2 or 3");
+  if (variant != 0 && variant != 1) return fail("unipc_coefficients: variant must be 0 (bh1) or 1 (bh2)");
+  for (int i = 0; i < n; ++i) {
+    if (ts[i] < 0 || ts[i] >= n_train) return fail("unipc_coefficients: timestep out of range [0, n_train)");
+    if (i > 0 && ts[i] >= ts[i - 1]) return fail("unipc_coefficients: timesteps must be strictly decreasing");
+    const double a = ac[ts[i]];
+    if (!(a > 0.0 && a < 1.0)) return fail("unipc_coefficients: alphas_cumprod[t] must lie in (0, 1)");
+  }
+  std::vector<double> al(n), sg(n), lam(n);
+  for (int i = 0; i < n; ++i) {
+    const double a = ac[ts[i]];
+    al[i] = sqrt(a);
+    sg[i] = sqrt(1.0 - a);
+    lam[i] = log(al[i] / sg[i]);
+  }
+  auto korder = [&](int i) { return std::min(order, std::min(i + 1, n - i)); };
+  for (int i = 0; i < n; ++i) {
+    double g = 0.0, a_c = 0.0, cm[4] = {0.0, 0.0, 0.0, 0.0}, a_p = 0.0, pm[3] = {0.0, 0.0, 0.0};
+    double phi1, Bh, b[3], r[3], rho[3];
+    if (i == 0) {
+      g = 1.0;
+    } else {
+      const int k = korder(i - 1);
+      const double h = lam[i] - lam[i - 1];
+      unipc_phi(h, variant, k, phi1, Bh, b);
+      for (int j = 1; j < k; ++j) r[j - 1] = (lam[i - 1 - j] - lam[i - 1]) / h;
+      r[k - 1] = 1.0;
+      if (k == 1)
+        rho[0] = 0.5;
+      else
+        unipc_solve(r, b, k, rho);
+      const double w = al[i] * Bh;
+      a_c = sg[i] / sg[i - 1];
+      cm[0] = -w * rho[k - 1];
+      cm[1] = -al[i] * phi1 + w * rho[k - 1];
+      for (int j = 1; j < k; ++j) {
+        cm[1] += w * rho[j - 1] / r[j - 1];
+        cm[1 + j] = -w * rho[j - 1] / r[j - 1];
+      }
+    }
+    if (i == n - 1) {
+      pm[0] = 1.0;  // to the clean sample: z' = m
+    } else {
+      const int k = korder(i);
+      const double h = lam[i + 1] - lam[i];
+      unipc_phi(h, variant, k, phi1, Bh, b);
+      for (int j = 1; j < k; ++j) r[j - 1] = (lam[i - j] - lam[i]) / h;
+      if (k == 2) rho[0] = 0.5;
+      if (k == 3) unipc_solve(r, b, 2, rho);
+      const double w = al[i + 1] * Bh;
+      a_p = sg[i + 1] / sg[i];
+      pm[0] = -al[i + 1] * phi1;
+      for (int j = 1; j < k; ++j) {
+        pm[0] += w * rho[j - 1] / r[j - 1];
+        pm[j] = -w * rho[j - 1] / r[j - 1];
+      }
+    }
+    const double row[16] = {sg[i], al[i], g,     a_c,   cm[0], cm[1], cm[2], cm[3],
+                            a_p,   pm[0], pm[1], pm[2], 10.0,  0.0,   0.0,   0.0};
+    for (int j = 0; j < 16; ++j) rows[(size_t)i * 16 + j] = (float)row[j];
+  }
+  return 0;
+}
+
+int UNet::unipc_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                       const long long* timesteps, int n, const float* ac, int n_train, int order, int variant,
+                       int* nan_flag, cudaStream_t st) {
+  if (n < 1 || n > 4096) return fail("unipc_sample: 1 <= n <= 4096 timesteps");
+  std::vector<float> coef((size_t)n * 16);
+  if (unipc_coefficients(timesteps, n, ac, n_train, order, variant, coef.data())) return -1;
+  if (sampler_begin(z_init, cond, B, T, h, w, st)) return -1;
+  UProgram* up = active;
+  if (!up->unipc_xc) {  // first use of this program: the buffers the captured graph will read
+    float* buf = (float*)up->ds.alloc(up->numel * 4 * 5);
+    if (!buf) return fail("out of device memory (UniPC state and history buffers)");
+    up->unipc_xc = buf;
+    up->unipc_hist = buf + up->numel;
+  }
+  if (loop_tables(*this, up, std::vector<long long>(timesteps, timesteps + n), coef, 16, st)) return -1;
+  if (loop_replay(*this, up, SAMPLER_UNIPC, 0, n, nullptr, 0, st)) return -1;
+  B2V_CUDA(cudaMemcpyAsync(z_out, up->x_in, up->numel * 4, cudaMemcpyDeviceToDevice, st));
+  if (nan_flag) B2V_CUDA(cudaMemcpyAsync(nan_flag, up->nan_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
+  return check_launches("unipc_sample");
 }
 
 // GaussianDiffusion.p_sample_loop (models/diffusion.py:340-367) as one graph replay per step.  coef: HOST rows indexed
@@ -798,7 +944,7 @@ int UNet::ddpm_run(const float* coef, int n, int first, int count, const float* 
       ts[s] = n - 1 - s;
       for (int j = 0; j < 8; ++j) rows[(size_t)s * 8 + j] = coef[(size_t)(n - 1 - s) * 8 + j];
     }
-    if (loop_tables(*this, up, ts, rows, st)) return -1;
+    if (loop_tables(*this, up, ts, rows, 8, st)) return -1;
     up->loop_n = n;
   } else if (n != up->loop_n) {
     return fail("ddpm_run: loop length changed between chunks");

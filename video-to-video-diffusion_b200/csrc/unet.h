@@ -27,7 +27,8 @@ struct ULevel {
   bool has_resample = false;
 };
 
-enum { SAMPLER_DDIM = 0, SAMPLER_DDPM = 1, SAMPLER_DPMPP = 2, SAMPLER_KINDS = 3 };  // as b2v_sampler_cfg.sampler
+// loop programs; b2v_sampler_cfg.sampler 0, 1 map to DDIM, DDPM, 2 and 3 to DPMPP, 4 to UNIPC
+enum { SAMPLER_DDIM = 0, SAMPLER_DDPM = 1, SAMPLER_DPMPP = 2, SAMPLER_UNIPC = 3, SAMPLER_KINDS = 4 };
 struct UProgram {
   int B = 0, T = 0, h = 0, w = 0;
   long long numel = 0;
@@ -37,6 +38,9 @@ struct UProgram {
   Program fwd, loop[SAMPLER_KINDS];  // one U-Net evaluation | per sampler: core without time_embed + update + advance
   float *x_in = nullptr, *c_in = nullptr, *eps = nullptr;
   float* x0_prev = nullptr;  // previous step's data prediction (DPM-Solver++), allocated by the first dpmpp_sample
+  // UniPC: the corrected state and the 4-slot ring of data predictions ([4][numel], slot = step % 4), allocated
+  // together ([5][numel]) by the first unipc_sample
+  float *unipc_xc = nullptr, *unipc_hist = nullptr;
   long long *t_dev = nullptr, *t_table = nullptr;
   SamplerCtl* ctl = nullptr;  // device loop state of the sampler graphs (step counter, NaN flag, noise source)
   int *step_dev = nullptr, *nan_dev = nullptr;  // = &ctl->step, &ctl->nan_flag
@@ -85,6 +89,10 @@ struct UNet {
   int dpmpp_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
                    const long long* timesteps, int n, const float* ac, int n_train, int order, int sde,
                    const float* noise, int* nan_flag, cudaStream_t st);
+  // UniPC over the timesteps (rows from unipc_coefficients; variant 0 = bh1, 1 = bh2)
+  int unipc_sample(const float* z_init, const float* cond, float* z_out, int B, int T, int h, int w,
+                   const long long* timesteps, int n, const float* ac, int n_train, int order, int variant,
+                   int* nan_flag, cudaStream_t st);
   int ddpm_step(long long t, const float* coef, const float* noise, cudaStream_t st);
   // loop steps [first, first + count) of an n-step ancestral loop (step s handles timestep n-1-s)
   int ddpm_run(const float* coef, int n, int first, int count, const float* noise, unsigned long long seed,
@@ -97,6 +105,9 @@ struct UNet {
 
 // host fp64 coefficient rows of DPM-Solver++(2M) (see b2v_dpmpp_coefficients); no device needed
 int dpmpp_coefficients(const long long* timesteps, int n, const float* ac, int n_train, int order, int sde,
+                       float* rows);
+// host fp64 coefficient rows [n][16] of UniPC (see b2v_unipc_coefficients); no device needed
+int unipc_coefficients(const long long* timesteps, int n, const float* ac, int n_train, int order, int variant,
                        float* rows);
 
 }  // namespace b2v

@@ -11,7 +11,7 @@ import torch
 
 from .. import _lib
 
-SAMPLERS = {"ddim": 0, "ddpm": 1, "dpmpp_2m": 2, "dpmpp_2m_sde": 3}
+SAMPLERS = {"ddim": 0, "ddpm": 1, "dpmpp_2m": 2, "dpmpp_2m_sde": 3, "unipc": 4}
 
 
 @torch.no_grad()
@@ -19,7 +19,8 @@ def generate_ensemble(model, v_in, sampler, num_inference_steps=20, num_samples=
                       return_members=False):
     """thick slices v_in (B, C, T_in, H, W) -> (mean, std), each (B, C, T_out, H, W) fp32, over K = num_samples samples
     per input; std is the unbiased per-voxel standard deviation (like torch.std).  With return_members=True also the
-    members (K, B, C, T_out, H, W).  sampler: "ddim" (eta = 0, as generate()), "ddpm", "dpmpp_2m" or "dpmpp_2m_sde".
+    members (K, B, C, T_out, H, W).  sampler: "ddim" (eta = 0, as generate()), "ddpm", "dpmpp_2m", "dpmpp_2m_sde" or
+    "unipc" (UniPC-3, bh2, as generate()).
 
     RNG order: z_init = torch.randn((K*B, L, T_out, H/4, W/4)); then for "dpmpp_2m_sde" one randn of that shape per step,
     for "ddpm" one seed = torch.randint(0, 2**62, ()) that keys the device Philox generator of the per-step noise.
@@ -63,6 +64,7 @@ def generate_ensemble(model, v_in, sampler, num_inference_steps=20, num_samples=
         ts, acp = _schedule(model.diffusion, num_inference_steps)
         keep += [ts, acp]
         cfg.n, cfg.n_train, cfg.eta = len(ts), acp.numel(), 0.0
+        cfg.unipc_order, cfg.unipc_variant = 3, 1  # read only for "unipc"
         cfg.timesteps = ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
         cfg.alphas_cumprod = ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float))
         if sampler == "dpmpp_2m_sde":

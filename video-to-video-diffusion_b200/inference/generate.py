@@ -1,9 +1,10 @@
 """Mirror of the tensor-level helper of the reference `inference/generate.py` (generate_batch, :98-155).
 The file-level helpers of the reference (mp4 decode/encode through cv2 / PyAV) are data I/O and out of scope.
-Besides the reference's "ddim" / "ddpm", sampler_type accepts "dpmpp_2m" and "dpmpp_2m_sde" (DPMSolverSampler)."""
+Besides the reference's "ddim" / "ddpm", sampler_type accepts "dpmpp_2m" and "dpmpp_2m_sde" (DPMSolverSampler) and
+"unipc" (UniPCSampler, order 3, bh2)."""
 import torch
 
-from .sampler import DDIMSampler, DDPMSampler, DPMSolverSampler
+from .sampler import DDIMSampler, DDPMSampler, DPMSolverSampler, UniPCSampler
 
 
 def generate_batch(model, input_videos, sampler_type="ddim", num_inference_steps=20, device="cuda"):
@@ -22,6 +23,9 @@ def generate_batch(model, input_videos, sampler_type="ddim", num_inference_steps
         z_0 = DPMSolverSampler(model.diffusion, model.unet).sample(z_in.shape, z_in, num_inference_steps, device,
                                                                     stochastic=sampler_type == "dpmpp_2m_sde",
                                                                     progress=True)
+    elif sampler_type == "unipc":
+        z_0 = UniPCSampler(model.diffusion, model.unet).sample(z_in.shape, z_in, num_inference_steps, device,
+                                                                progress=True)
     else:
         raise ValueError(f"Unknown sampler type: {sampler_type}")
     with torch.no_grad():

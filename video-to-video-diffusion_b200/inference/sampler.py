@@ -44,9 +44,9 @@ def _schedule(diffusion, num_inference_steps):
     return ts, diffusion.alphas_cumprod.detach().float().cpu().contiguous()
 
 
-def _native_sample(smp, entry, shape, conditioning, device, ts, acp, args, draw_noise):
+def _native_sample(smp, entry, shape, conditioning, device, ts, acp, args, draw_noise, takes_noise=True):
     """the whole loop as one call of b2v_<entry> on a native UNet3D; RNG order: z, then one randn_like per step if
-    draw_noise.  args are the entry's own arguments between n_train and noise."""
+    draw_noise.  args are the entry's own arguments between n_train and noise (nan_flag when not takes_noise)."""
     shape, dev = check_sampler_args(smp.model, shape, conditioning, device)  # ValueError before any C call
     z = torch.randn(shape, device=dev)
     cond = conditioning.detach().to(dev, torch.float32).contiguous()
@@ -62,7 +62,7 @@ def _native_sample(smp, entry, shape, conditioning, device, ts, acp, args, draw_
             smp.model.native(dev), _lib.dptr(z), _lib.dptr(cond), _lib.dptr(out), B, T, h, w,
             ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), n,
             ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)), acp.numel(), *args,
-            _lib.dptr(noise), _lib.dptr(flag, torch.int32), _lib.stream()), entry)
+            *((_lib.dptr(noise),) if takes_noise else ()), _lib.dptr(flag, torch.int32), _lib.stream()), entry)
     smp.last_nan_flag = flag  # device tensor; .item() it to learn whether a NaN/Inf guard fired
     return out
 
@@ -226,6 +226,81 @@ class DPMSolverSampler(_Stitching):
         return self._stitch(v_thick_full, vae,
                             lambda s, c: self.sample(s, c, num_inference_steps, device, order=order,
                                                      stochastic=stochastic, progress=False),
+                            patch_size, target_patch_size, stride, device)
+
+
+UNIPC_VARIANTS = {"bh1": 0, "bh2": 1}
+
+
+def unipc_coefficients(timesteps, alphas_cumprod, order=3, variant="bh2"):
+    """the (n, 16) fp32 rows {sigma, alpha, g, a_c, c0..c3, a_p, p0..p2, clip, 0, 0, 0} of a UniPC loop over `timesteps`
+    (strictly decreasing), computed in fp64 by b2v_unipc_coefficients (host only, no device needed)"""
+    if variant not in UNIPC_VARIANTS:
+        raise ValueError(f"unipc_coefficients: variant must be 'bh1' or 'bh2', got {variant!r}")
+    ts = np.ascontiguousarray(timesteps, dtype=np.int64)
+    acp = alphas_cumprod.detach().float().cpu().contiguous()
+    rows = torch.empty((len(ts), 16), dtype=torch.float32)
+    _lib.check(_lib.lib().b2v_unipc_coefficients(
+        ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), len(ts), ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float)),
+        acp.numel(), int(order), UNIPC_VARIANTS[variant], ctypes.cast(rows.data_ptr(), ctypes.POINTER(ctypes.c_float))),
+        "unipc_coefficients")
+    return rows
+
+
+class UniPCSampler(_Stitching):
+    """UniPC (Zhao et al. 2023), not in the reference: a predictor-corrector multistep solver over the same
+    eps-prediction U-Net.  The corrector reuses the evaluation the next step needs anyway, so a predictor of order p
+    becomes a solver of order p + 1 at one U-Net evaluation per step, like DDIM, over DDIMSampler's timestep subset.
+    order 3 with variant "bh2" (the default, and generate(sampler="unipc")) is the choice for guidance-free sampling from
+    about 10 steps up; below 10 steps order=1 is more accurate.  With a native UNet3D the whole loop is one call
+    (b2v_unipc_sample); any other callable model runs a Python loop over the same update kernel.  RNG order: z =
+    randn(shape), nothing else (deterministic solver)."""
+
+    def __init__(self, diffusion, model):
+        self.diffusion, self.model, self.timesteps = diffusion, model, diffusion.timesteps
+
+    def _get_timesteps(self, num_inference_steps):
+        return _timesteps(self.timesteps, num_inference_steps)
+
+    @torch.no_grad()
+    def sample(self, shape, conditioning, num_inference_steps, device, order=3, variant="bh2", progress=True):
+        if order not in (1, 2, 3):
+            raise ValueError(f"UniPCSampler: order must be 1, 2 or 3, got {order}")
+        if variant not in UNIPC_VARIANTS:
+            raise ValueError(f"UniPCSampler: variant must be 'bh1' or 'bh2', got {variant!r}")
+        ts, acp = _schedule(self.diffusion, num_inference_steps)
+        if _is_native(self.model):
+            return _native_sample(self, "unipc_sample", shape, conditioning, device, ts, acp,
+                                  (int(order), UNIPC_VARIANTS[variant]), False, takes_noise=False)
+        dev = torch.device(device)
+        z = torch.randn(shape, device=dev)
+        cond = conditioning.detach().to(dev, torch.float32).contiguous()
+        if z.numel() == 0:
+            return z
+        return self._sample_generic(z, cond, ts, unipc_coefficients(ts, acp, order, variant).to(dev))
+
+    def _sample_generic(self, z, cond, ts, rows):
+        """any callable model(z, t, c): Python loop, the update kernel per step (in place on z)"""
+        dev = z.device
+        xc = torch.empty_like(z)
+        hist = torch.empty((4,) + tuple(z.shape), dtype=torch.float32, device=dev)
+        flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        for i, t_idx in enumerate(ts):
+            t = torch.full((z.shape[0],), int(t_idx), device=dev, dtype=torch.long)
+            eps = self.model(z, t, cond).float().contiguous()
+            flag |= ops.unipc_update(z, xc, hist, eps, rows[i].contiguous(), i)
+        self.last_nan_flag = flag
+        return z
+
+    @torch.no_grad()
+    def sample_with_stitching(self, v_thick_full, vae, num_inference_steps: int = 20,
+                              patch_size: Tuple[int, int, int] = (8, 192, 192),
+                              target_patch_size: Tuple[int, int, int] = (48, 192, 192),
+                              stride: Tuple[int, int, int] = (4, 96, 96), device="cuda", order=3, variant="bh2",
+                              progress=True):
+        return self._stitch(v_thick_full, vae,
+                            lambda s, c: self.sample(s, c, num_inference_steps, device, order=order, variant=variant,
+                                                     progress=False),
                             patch_size, target_patch_size, stride, device)
 
 

@@ -1,7 +1,7 @@
 """Mirror of the reference `models/model.py` facade: `VideoToVideoDiffusion(config)` resolves the config the way
 the reference does (including reading the U-Net keys from the top level of the dict only), exposes `.vae`, `.unet`,
 `.diffusion` under the same names so reference checkpoints load, and `generate()` runs
-encode -> depth upsample -> DDIM/DDPM (or DPM-Solver++(2M), not in the reference) -> decode entirely on libb2v.so.  Training (`forward`, `save_checkpoint`)
+encode -> depth upsample -> DDIM/DDPM (or DPM-Solver++(2M) or UniPC, not in the reference) -> decode entirely on libb2v.so.  Training (`forward`, `save_checkpoint`)
 is out of scope of this package.
 """
 import ctypes
@@ -77,8 +77,9 @@ class VideoToVideoDiffusion(nn.Module):
     def generate(self, v_in, sampler, num_inference_steps=20, guidance_scale=1.0, target_depth=None):
         """thick slices (B,C,T_in,H,W) -> thin slices (B,C,T_out,H,W), fp32, tanh-bounded.  `guidance_scale` is
         accepted and ignored, exactly like the reference.  Besides the reference's "ddim" / "ddpm", `sampler` may be
-        "dpmpp_2m" or "dpmpp_2m_sde" (DPM-Solver++(2M), ODE / SDE: num_inference_steps as for DDIM)."""
-        if sampler not in ("ddpm", "ddim", "dpmpp_2m", "dpmpp_2m_sde"):
+        "dpmpp_2m" or "dpmpp_2m_sde" (DPM-Solver++(2M), ODE / SDE) or "unipc" (UniPC-3, bh2), num_inference_steps as for
+        DDIM."""
+        if sampler not in ("ddpm", "ddim", "dpmpp_2m", "dpmpp_2m_sde", "unipc"):
             raise ValueError(f"Unknown sampler: {sampler}")
         device = v_in.device
         B, C, T_in, H, W = v_in.shape
@@ -105,8 +106,9 @@ class VideoToVideoDiffusion(nn.Module):
             from ..inference.sampler import _schedule
             ts, acp = _schedule(self.diffusion, num_inference_steps)
             keep += [ts, acp]
-            code = {"ddim": 0, "dpmpp_2m": 2, "dpmpp_2m_sde": 3}[sampler]
+            code = {"ddim": 0, "dpmpp_2m": 2, "dpmpp_2m_sde": 3, "unipc": 4}[sampler]
             cfg.sampler, cfg.n, cfg.n_train, cfg.eta = code, len(ts), acp.numel(), 0.0
+            cfg.unipc_order, cfg.unipc_variant = 3, 1  # UniPC-3, bh2 (read only for code 4)
             cfg.timesteps = ts.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
             cfg.alphas_cumprod = ctypes.cast(acp.data_ptr(), ctypes.POINTER(ctypes.c_float))
             if sampler == "dpmpp_2m_sde":

@@ -146,6 +146,20 @@ def dpmpp_update(z, x0_prev, eps, coef, noise=None):
     return flag
 
 
+def unipc_update(z, xc, hist, eps, coef, step):
+    """in-place UniPC step `step` of a loop (fp32): z (the evaluated state) becomes the next state, xc the corrected
+    state, hist[step % 4] the data prediction m_step; hist is the (4,) + z.shape ring of data predictions, read at
+    slots (step - j) % 4 only where the row's weights are non-zero; coef: device fp32[16], one b2v_unipc_coefficients
+    row.  Returns the NaN flag tensor."""
+    if tuple(hist.shape) != (4,) + tuple(z.shape):
+        raise ValueError(f"unipc_update: hist must have shape (4,) + {tuple(z.shape)}, got {tuple(hist.shape)}")
+    flag = torch.zeros(1, dtype=torch.int32, device=z.device)
+    _lib.check(_lib.lib().b2v_unipc_update(_lib.dptr(z), _lib.dptr(xc), _lib.dptr(hist), _lib.dptr(eps), _lib.dptr(coef),
+                                           int(step), z.numel(), _lib.dptr(flag, torch.int32), _lib.stream()),
+               "unipc_update")
+    return flag
+
+
 def ddpm_update(z, eps, noise, coef_row):
     """in-place DDPM ancestral update of z (fp32); coef_row: 8 host floats (GaussianDiffusion.ddpm_coefficients()[t])"""
     coef = (ctypes.c_float * 8)(*[float(v) for v in coef_row])
